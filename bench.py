@@ -424,6 +424,8 @@ def run_silk(args):
         tc = O.lib().orc_silk_bench(O.ptr(sample), ns, nfr, nb, 2, 20, ch, cores, None, ctypes.byref(x))
         cpu = {"value": ns * nfr / tc * FRAME_S, "unit": "streams", "cores": cores, "kind": "port",
                "sample": f"{nfr} chained frames x {ns} streams of the same packets, C oracle (oracle/silk.c), one thread per core, {tc:.2f} s wall"}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, dec, n, n48, ch, dev)
     if rank == 0:
         peak, peak_src = measured_peak_gbs()
         chan_frames = n * ch
@@ -478,6 +480,37 @@ def emit(line):
     out.flush()
 
 
+DUMP_BYTES = 64_000_000  # array data written by --dump-outputs at most
+
+
+class _DeviceArray:
+    """A device pointer the library hands out, in the form torch.as_tensor reads (__cuda_array_interface__)."""
+
+    def __init__(self, ptr, shape, typestr):
+        self.__cuda_array_interface__ = {"data": (ptr, False), "shape": shape, "typestr": typestr, "version": 2}
+
+
+def dump_outputs(out_dir, dec, n, frame, channels, dev):
+    """--dump-outputs: what a caller of the device-resident path receives after the last timed step, as .npy files:
+    pcm [streams, frame * channels] float32 (interleaved; read from the decoder's PCM ring, where the step's frame ends at
+    each stream's ring position), final_range [streams] (the range coder's final state per stream, exact in float64) and
+    stream [streams] (stream ids).  Above DUMP_BYTES a fixed, seeded sample of the streams is written."""
+    import torch
+    per_stream = frame * channels * 4 + 8 + 8
+    k = min(n, DUMP_BYTES // per_stream)
+    ids = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    ring_ptr, ring_n, pos_ptr = dec.ring()
+    ring = torch.as_tensor(_DeviceArray(ring_ptr, (n, ring_n, channels), "<f4"), device=dev)
+    pos = torch.as_tensor(_DeviceArray(pos_ptr, (n,), "<i4"), device=dev).long()
+    sel = torch.from_numpy(ids).to(dev)
+    idx = (pos[sel, None] - frame + torch.arange(frame, device=dev)) % ring_n
+    pcm = torch.gather(ring[sel], 1, idx[:, :, None].expand(-1, -1, channels)).reshape(k, frame * channels)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pcm.npy"), pcm.cpu().numpy())
+    np.save(os.path.join(out_dir, "final_range.npy"), dec.final_ranges()[ids].astype(np.float64))
+    np.save(os.path.join(out_dir, "stream.npy"), ids.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -493,8 +526,13 @@ def main():
                     help="extra workload: per-packet frame sizes 2.5-20 ms with transients, device-resident (BASELINE configs[4] shape, CELT part)")
     ap.add_argument("--silk", action="store_true",
                     help="extra workload: BASELINE configs[2], SILK-only wideband 20 ms mono streams (SYNTH-SILK/1), default 16384 streams")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write the last step's outputs (PCM, final range per stream) as DIR/<name>.npy, "
+                         "rank 0; the inputs are the same in every run with the same arguments")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
+    if args.dump_outputs and (args.mix or args.impl != "b200"):
+        raise SystemExit("--dump-outputs covers the b200 arm's fixed-frame workloads (the default and --silk)")
     quiet_stdout()
     if args.silk:
         if args.impl != "b200":
@@ -726,6 +764,8 @@ def main():
                "sample": f"{reps} passes over {fr} chained frames x {n} streams of the same packets, C oracle port of the reference crate "
                          f"(range decode + PVQ + IMDCT + comb filter), one thread per core, {tc:.1f} s wall"}
 
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, dec, n, NF, CHANNELS, dev)
     if rank == 0:
         peak, peak_src = measured_peak_gbs()
         ch_frames = n * CHANNELS

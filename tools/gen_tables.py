@@ -2,8 +2,8 @@
 """Generate the constant tables of the CELT 48 kHz / 960 standard mode.
 
 Nothing here is copied from the reference: every table is recomputed from its
-defining formula and the result is checked (tests/test_tables_vs_reference.py,
-container-only) against the literals in the reference crate:
+defining formula and the result is checked (tests/test_tables_vs_reference.py)
+against the literals in the reference crate, kept in tests/golden/reference_tables.json:
 
   TRIG[1800]      /root/reference/src/celt/mdct.rs:265-626
                   f32(cos(2*PI_F*(i+1/8)/N)) for N = 1920, 960, 480, 240 (i < N/2), where
