@@ -188,8 +188,9 @@ int opn_batch_ring(opn_batch *b, float **ring, uint32_t *ring_samples, uint32_t 
 /* Counters for the measurement harness.  kernel_ms[k]/kernel_launches[k]: k = 0 range decode (k_synth_rangedec),
  * 1 frame kernel (k_frame_w: PVQ expansion + IMDCT + TDAC + comb post-filter + PCM store; a large batch runs it as three
  * concurrent launches over thirds of the streams, and kernel_ms[1] is the time from the first launch to the last
- * completion), 2 stand-alone PVQ expansion (only in the unfused variant, OPN_UNFUSED_EXPAND=1).  Timing must be enabled
- * first (the stages of a step then run one after the other, with cudaEvents around each). */
+ * completion), 2 the two bucketing kernels of a mixed-frame step (k_mix_key, k_mix_place: counted, not timed; kernel_ms[2]
+ * stays 0).  Timing must be enabled first (the stages of a step then run one after the other, with cudaEvents around
+ * each). */
 int opn_batch_enable_timing(opn_batch *b, int on);
 int opn_batch_stats(opn_batch *b, uint64_t kernel_launches[3], double kernel_ms[3], int reset);
 /* Sum over the channel-frames the post-filter ran on, in timed passes, of max(T0,T1)+2: the history samples it had to

@@ -8,11 +8,8 @@
 // (comb_filter_inplace, src/celt/comb_filter/mod.rs:130-193, scalar kernel fallback.rs:32-53) runs on those rows
 // before the only PCM store.  The post-filter's history -- the previous max(T0,T1)+2 output samples -- is the PCM ring
 // itself: taps that fall before the frame are read from the ring through L1/L2 (one float2 = both channels of a
-// sample), taps inside the frame from the rows.  Shared memory per stream: C rows of nf+60 floats and one mbarrier
+// sample), taps inside the frame from the rows.  Shared memory per stream: C rows of nf+60 floats and a small stash
 // (8 KB for a stereo 20 ms frame), as for the IMDCT alone.
-//
-// A variant of the same kernel (EXPAND = false) takes its coefficient rows from global memory by TMA instead
-// (unfused pipeline, kept for measurements).
 #pragma once
 #include "imdct_warp.cuh"
 #include "symbols.cuh"
@@ -219,7 +216,7 @@ constexpr int FRAME_WARPS = OPN_FRAME_WARPS, FRAME_CTAS = OPN_FRAME_CTAS;
 #define OPN_STORE_UNROLL 3  // 15 (the whole loop) measured 1-2 % slower per step: the kernel is sensitive to its code size
 #endif
 constexpr int STORE_UNROLL = OPN_STORE_UNROLL;  // iterations of the PCM store loop in flight
-// per warp: the rows, 16 bytes for an mbarrier (coefficient rows by TMA) and a 48-byte stash (frame header, previous
+// per warp: the rows, 16 bytes of padding (the layout the kernel was tuned with) and a 48-byte stash (frame header, previous
 // post-filter parameters, ring position: read once in the prologue, used again after the transform)
 __host__ __device__ constexpr size_t frame_warp_bytes(int lm, int channels) { return (size_t)channels * w_ch_floats(lm) * 4 + 16 + 48; }
 __host__ __device__ constexpr size_t frame_smem_bytes(int lm, int channels, size_t blob_bytes)
@@ -227,9 +224,9 @@ __host__ __device__ constexpr size_t frame_smem_bytes(int lm, int channels, size
     return 16 + blob_bytes + (size_t)FRAME_WARPS * frame_warp_bytes(lm, channels);
 }
 
-// MODE: where the coefficient rows come from.  FRAME_ROWS: global memory, by TMA (unfused variant); FRAME_SYNTH1: expanded from
-// the codeword indices of the static SYNTH-CELT/1 schedule; FRAME_SYNTH2: expanded from the per-frame part list of SYNTH-CELT/2.
-enum { FRAME_ROWS = 0, FRAME_SYNTH1 = 1, FRAME_SYNTH2 = 2 };
+// MODE: where the coefficient rows come from.  FRAME_SYNTH1: expanded from the codeword indices of the static SYNTH-CELT/1
+// schedule; FRAME_SYNTH2: expanded from the per-frame part list of SYNTH-CELT/2.
+enum { FRAME_SYNTH1 = 1, FRAME_SYNTH2 = 2 };
 // One CTA of the frame kernel: its FRAME_WARPS warps take the items first_item .. first_item + FRAME_WARPS - 1 (< item_end).
 // CS: channels of the PACKETS (the crate's stream_channels, decoder.rs:332,376,395), C: channels of the decoder.  They
 // differ when a mono packet reaches a stereo decoder or the reverse; the frame is then expanded with the packet's layout
@@ -239,9 +236,7 @@ enum { FRAME_ROWS = 0, FRAME_SYNTH1 = 1, FRAME_SYNTH2 = 2 };
 template <int LM, int C, int MODE, int CS = C>
 __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_item, uint32_t item_end)
 {
-    constexpr bool EXPAND = MODE != FRAME_ROWS;
     constexpr int R = C > CS ? C : CS;  // rows of shared memory per stream
-    static_assert(EXPAND || CS == C, "coefficient rows from memory are the decoder's channels already");
     extern __shared__ __align__(16) uint8_t smem[];
     constexpr int NF = 120 << LM;
     constexpr int CHF = w_ch_floats(LM);
@@ -250,7 +245,6 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
     const uint8_t *blob = smem + 16;
     const FBlobHdr H = g_tab.fblob_hdr[LM][CS - 1];  // the schedule's tables are the packet layout's; the transform's are the same in both
     float *o = reinterpret_cast<float *>(smem + 16 + H.total + (size_t)warp * frame_warp_bytes(LM, R));
-    uint64_t *bar = reinterpret_cast<uint64_t *>(o + R * CHF);  // this warp's barrier (coefficient rows by TMA, unfused variant)
     uint4 *stash = reinterpret_cast<uint4 *>(o + R * CHF + 4);  // [0] frame header, [1] previous PfState, [2].x ring position
 
     if (threadIdx.x == 0) {
@@ -261,15 +255,6 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
     const uint32_t item = first_item + warp;
     const bool in_range = item < item_end;
     const uint32_t stream = in_range ? (A.stream_idx ? A.stream_idx[item] : item) : 0u;
-    if constexpr (!EXPAND) {
-        // coefficient rows -> output rows by TMA, before anything else (the row address only needs `stream`)
-        if (lane == 0 && in_range) {
-            mbar_init(bar, 1);
-            mbar_expect_tx(bar, C * NF * 4);
-#pragma unroll
-            for (int c = 0; c < C; c++) bulk_g2s(o + c * CHF, A.coef + ((size_t)stream * C + c) * NF, NF * 4, bar);
-        }
-    }
     // What the transform needs is loaded now; the rest of the post-filter state is read after the transform, so that it
     // does not occupy registers across it (its cache lines are already here by then).
     const int32_t status = in_range ? A.status[stream] : -1;
@@ -314,19 +299,14 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
             prefetch_l2(ring + (size_t)j * C);
         }
     }
-    if constexpr (EXPAND) {
-        // the coefficient rows start out zero: w_expand only writes the pulses
+    // the coefficient rows start out zero: w_expand only writes the pulses
 #pragma unroll
-        for (int c = 0; c < R; c++)
-            for (int i = lane; i < NF / 4; i += 32) reinterpret_cast<float4 *>(o + c * CHF)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
+    for (int c = 0; c < R; c++)
+        for (int i = lane; i < NF / 4; i += 32) reinterpret_cast<float4 *>(o + c * CHF)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     __syncthreads();  // the table barrier is initialised
     mbar_wait(tbar, 0);
     if (status < 0) {  // out of range, or a rejected packet: state untouched (decoder.rs:397)
         if (in_range && lane == 0 && A.result) A.result[stream] = status;
-        if constexpr (!EXPAND) {
-            if (in_range) mbar_wait(bar, 0);  // the rows are in flight: do not retire the CTA under them
-        }
         return;
     }
     const float2 *t_long = reinterpret_cast<const float2 *>(blob + H.tp_long), *t_short = reinterpret_cast<const float2 *>(blob + H.tp_short);
@@ -354,8 +334,6 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
             w_expand2<CS>(T, LM, (uint32_t)lane, A.parts + (size_t)stream * CELT2_MAX_PARTS, stash[0].w, A.bande + (size_t)stream * 42, o, CHF, nullptr, lmt);
         }
         __syncwarp();
-    } else {
-        mbar_wait(bar, 0);
     }
     if constexpr (CS == 1 && C == 2) {  // mono packet, stereo decoder: both channels transform the same spectrum
         for (int i = lane; i < NF / 4; i += 32) reinterpret_cast<float4 *>(o + CHF)[i] = reinterpret_cast<const float4 *>(o)[i];
@@ -368,7 +346,7 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
         __syncwarp();
     }
     if constexpr (LM > 0) {
-        if ((hdr_x >> 2) & 1u) w_imdct<3, (1 << LM), C, true, EXPAND>(o, lane, carry, t_short, t_tw, t_win);  // expanded rows are block-major
+        if ((hdr_x >> 2) & 1u) w_imdct<3, (1 << LM), C, true, true>(o, lane, carry, t_short, t_tw, t_win);  // expanded rows are block-major
         else w_imdct<3 - LM, 1, C, true>(o, lane, carry, t_long, t_tw, t_win);
     } else {
         w_imdct<3, 1, C, true>(o, lane, carry, t_long, t_tw, t_win);

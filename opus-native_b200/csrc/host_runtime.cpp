@@ -8,7 +8,6 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <string>
@@ -133,7 +132,7 @@ struct opn_batch {
 #endif
     static constexpr int NSETS = OPN_NSETS, NRD = OPN_NRD;
     cudaStream_t stream_rd[NRD] = {};     // set p decodes on stream_rd[p % NRD]: entropy stages of NRD steps overlap each other
-    cudaStream_t stream_ex = nullptr;     // unfused variant only: stand-alone PVQ expansion between the entropy streams and `stream`
+    cudaStream_t stream_mix = nullptr;    // bucketing of mixed-frame steps (k_mix_key / k_mix_place), ahead of their range decodes
     // A large bucket's frame kernel is cut into NGROUPS launches over contiguous stream ranges, group g on stream_fr[g]
     // (stream_fr[0] is `stream`).  A stream's frames stay in order (its group's stream), but the tail of one group's launch
     // overlaps the body of the other's, and step n+1 of a group may start while step n of the other is still running:
@@ -143,26 +142,23 @@ struct opn_batch {
 #define OPN_FRAME_GROUPS 3
 #endif
     static constexpr int NGROUPS = OPN_FRAME_GROUPS;
-    static constexpr uint32_t GROUP_MIN_ITEMS = 2048;  // smaller buckets run as one launch on `stream`
+    static constexpr uint32_t GROUP_MIN_ITEMS = 2048;  // smaller batches run the frame kernel as one launch on `stream`
     cudaStream_t stream_fr[NGROUPS] = {};
     cudaEvent_t ev_fr[NSETS][NGROUPS] = {};  // frame kernel of set p, group g finished
     cudaEvent_t ev_sw = nullptr;             // mode switch: everything enqueued on `stream` so far
-    cudaEvent_t ev_tm[NGROUPS] = {};         // timed pass: group g's launch finished
     bool fr_pending[NGROUPS] = {};           // group g >= 1 has work that `stream` has not been ordered after yet
     int fr_last_set[NGROUPS] = {};
     cudaEvent_t ev_k1[NSETS] = {};        // frame kernel(s) of set p finished on `stream` (group 0 / ungrouped): the set is free again
     bool k1_recorded[NSETS] = {};
     bool k1_grouped[NSETS] = {};          // set p was last used by a grouped launch: ev_fr[p][1..] are part of "set p is free"
     cudaEvent_t ev_rd[NSETS] = {};        // range decode of set p finished
-    cudaEvent_t ev_ex[NSETS] = {};        // unfused variant: coefficients of set p ready
     cudaEvent_t ev_in = nullptr;          // inputs ordered on `stream` / `stream_up` are complete
     static constexpr int MAX_CHUNKS = 8;
     cudaStream_t stream_up = nullptr, stream_dn = nullptr;  // host path: item/packet upload, PCM download
     cudaEvent_t ev_chunk[MAX_CHUNKS] = {};                  // frame kernels (and epilogue) of a chunk finished
     int set = 0;
-    bool unfused = false;  // OPN_UNFUSED_EXPAND=1 in the environment at creation: expansion as its own kernel, coefficient rows through HBM
     // per-stream state (device, SoA)
-    float *d_carry = nullptr, *d_ring = nullptr, *d_coef[NSETS] = {};
+    float *d_carry = nullptr, *d_ring = nullptr;
     uint32_t *d_ring_pos = nullptr, *d_final = nullptr, *d_idx[NSETS] = {};
     PfState *d_pf = nullptr;
     uint4 *d_hdr[NSETS] = {};
@@ -188,7 +184,7 @@ struct opn_batch {
     int stg_next = 0;
     float *d_softclip = nullptr;
     // mixed-frame steps (OPN_FLAG_MIXED_FRAMES), allocated on first use: the step's buckets are built on the device
-    // (k_mix_key / k_mix_place on stream_ex, in step order) into one item table + plan per buffer set
+    // (k_mix_key / k_mix_place on stream_mix, in step order) into one item table + plan per buffer set
     uint8_t *d_last_lm = nullptr, *d_mix_key = nullptr;  // [n] state: LM of the last decoded packet; scratch: bucket of the stream
     uint32_t *d_mix_rank = nullptr;                      // [n] scratch
     uint32_t *d_mix_items[NSETS] = {};                   // [3][mix_item_cap(n)]: offsets | lens | stream ids, by item
@@ -255,7 +251,9 @@ int batch_alloc_staging(opn_batch *b, opn_batch::Staging &g, size_t arena_bytes,
     return OPN_OK;
 }
 
-int timed_launch(opn_batch *b, int kind, cudaError_t (*fn)(opn_batch *, const void *), const void *args)
+// Runs `launch`, which enqueues one stage of a step.  In a timed pass the stage sits between two events on `stream`, so
+// whatever it enqueues on other streams must be joined back onto `stream` before it returns.
+template <class F> int timed_launch(opn_batch *b, int kind, F &&launch)
 {
     EventRing &r = b->ev[kind];
     if (b->timing) {
@@ -265,61 +263,14 @@ int timed_launch(opn_batch *b, int kind, cudaError_t (*fn)(opn_batch *, const vo
         }
         CU(cudaEventRecord(r.a[r.used], b->stream));
     }
-    CU(fn(b, args));
+    int rc = launch();
+    if (rc) return rc;
     if (b->timing) {
         CU(cudaEventRecord(r.b[r.used], b->stream));
         r.used++;
         r.launches++;
     }
-    b->launches[kind]++;
     return OPN_OK;
-}
-
-cudaError_t do_rangedec(opn_batch *b, const void *a)
-{
-    const SymbolArgs &s = *static_cast<const SymbolArgs *>(a);
-    return b->cfg.bitstream == OPN_BITSTREAM_SYNTH_CELT_2 ? launch_celt2_rangedec(s, b->stream) : launch_synth_rangedec(s, b->stream);
-}
-cudaError_t do_expand(opn_batch *b, const void *a) { return launch_synth_expand(*static_cast<const SymbolArgs *>(a), b->stream); }
-bool frame_grouped(const opn_batch *b, const FrameArgs &m)
-{
-    return !b->unfused && opn_batch::NGROUPS > 1 && m.n_items >= opn_batch::GROUP_MIN_ITEMS && !m.stream_idx;
-}
-// Timed pass: the frame kernel in its product configuration -- a large bucket as NGROUPS concurrent launches -- between
-// the two events timed_launch records on `stream` (the second one is ordered after every group).
-// streams [group_first(g), group_first(g + 1)) of an n-stream batch are group g of G (the same cut as a uniform bucket's item ranges)
-uint32_t group_first(uint32_t n, int g, int G) { return (uint32_t)((uint64_t)n * (uint32_t)g / (uint32_t)G); }
-int mix_groups(const opn_batch *b) { return (opn_batch::NGROUPS > 1 && b->n >= opn_batch::GROUP_MIN_ITEMS) ? opn_batch::NGROUPS : 1; }
-cudaError_t do_frame(opn_batch *b, const void *a)
-{
-    FrameArgs m = *static_cast<const FrameArgs *>(a);
-    if (m.plan) {  // mixed-frame step: one launch per group of the plan
-        const int G = mix_groups(b);
-        if (G == 1) return launch_frame_mix(m, b->n, b->stream);
-        cudaError_t e = cudaEventRecord(b->ev_sw, b->stream);
-        for (int g = 0; g < G && e == cudaSuccess; g++) {
-            cudaStream_t st = g == 0 ? b->stream : b->stream_fr[g];
-            if (g > 0) e = cudaStreamWaitEvent(st, b->ev_sw, 0);
-            m.group = g;
-            if (e == cudaSuccess) e = launch_frame_mix(m, group_first(b->n, g + 1, G) - group_first(b->n, g, G), st);
-            if (g > 0 && e == cudaSuccess) e = cudaEventRecord(b->ev_tm[g], st);
-            if (g > 0 && e == cudaSuccess) e = cudaStreamWaitEvent(b->stream, b->ev_tm[g], 0);
-        }
-        return e;
-    }
-    if (!frame_grouped(b, m)) return launch_frame(m, b->stream);
-    cudaError_t e = cudaEventRecord(b->ev_sw, b->stream);
-    const uint32_t n_items = m.n_items;
-    for (int g = 0; g < opn_batch::NGROUPS && e == cudaSuccess; g++) {
-        cudaStream_t st = g == 0 ? b->stream : b->stream_fr[g];
-        if (g > 0) e = cudaStreamWaitEvent(st, b->ev_sw, 0);
-        m.item0 = (uint32_t)((uint64_t)n_items * g / opn_batch::NGROUPS);
-        m.item_end = (uint32_t)((uint64_t)n_items * (g + 1) / opn_batch::NGROUPS);
-        if (e == cudaSuccess) e = launch_frame(m, st);
-        if (g > 0 && e == cudaSuccess) e = cudaEventRecord(b->ev_tm[g], st);
-        if (g > 0 && e == cudaSuccess) e = cudaStreamWaitEvent(b->stream, b->ev_tm[g], 0);
-    }
-    return e;
 }
 
 // Orders `stream` after everything the other frame groups have been given so far.
@@ -336,7 +287,7 @@ int join_groups(opn_batch *b)
 int sync_pipeline(opn_batch *b)
 {
     for (int q = 0; q < opn_batch::NRD; q++) CU(cudaStreamSynchronize(b->stream_rd[q]));
-    CU(cudaStreamSynchronize(b->stream_ex));
+    CU(cudaStreamSynchronize(b->stream_mix));
     for (int g = 1; g < opn_batch::NGROUPS; g++) {
         CU(cudaStreamSynchronize(b->stream_fr[g]));
         b->fr_pending[g] = false;
@@ -347,9 +298,104 @@ int sync_pipeline(opn_batch *b)
     return OPN_OK;
 }
 
-// One bucket = items of equal frame size that may run concurrently.
-// inputs_on: 0 = the packets are already complete in device memory (the entropy stage may start at once),
+// A timed pass runs every stage of a step in order on `stream`.
+cudaStream_t rd_stream(const opn_batch *b, int p) { return b->timing ? b->stream : b->stream_rd[p % opn_batch::NRD]; }
+cudaStream_t mix_stream(const opn_batch *b) { return b->timing ? b->stream : b->stream_mix; }
+
+// Makes `to` wait for everything enqueued on `from` so far.
+int order_after(cudaEvent_t ev, cudaStream_t from, cudaStream_t to)
+{
+    if (from == to) return OPN_OK;
+    CU(cudaEventRecord(ev, from));
+    CU(cudaStreamWaitEvent(to, ev, 0));
+    return OPN_OK;
+}
+
+// Start of a step: claims buffer set p and returns it (or an error).  The stream of the step's first kernel -- the
+// bucketing stream of a mixed-frame step, else the range-decode stream of set p -- is ordered after the step's inputs and
+// waits until set p is free again: the frame kernels of the step that used it last have finished.
+// inputs_on: 0 = the packets are already complete in device memory (the step may start at once),
 //            1 = they are ordered on b->stream, 2 = they are ordered on b->stream_up (host path).
+int begin_step(opn_batch *b, bool mixed, int inputs_on)
+{
+    const int p = b->set;
+    b->set = (p + 1) % opn_batch::NSETS;
+    const cudaStream_t first = mixed ? mix_stream(b) : rd_stream(b, p);
+    if (inputs_on) {
+        const int rc = order_after(b->ev_in, inputs_on == 1 ? b->stream : b->stream_up, first);
+        if (rc) return rc;
+    }
+    if (b->k1_recorded[p] && first != b->stream) {  // ev_k1[p] and the groups it joined are behind `stream` already
+        CU(cudaStreamWaitEvent(first, b->ev_k1[p], 0));
+        if (b->k1_grouped[p])
+            for (int g = 1; g < opn_batch::NGROUPS; g++) CU(cudaStreamWaitEvent(first, b->ev_fr[p][g], 0));
+    }
+    return p;
+}
+
+// The range decode of a step on buffer set p: launch(st) enqueues it on st; ev_rd[p] marks its end.
+template <class F> int range_decode(opn_batch *b, int p, F &&launch)
+{
+    const cudaStream_t srd = rd_stream(b, p);
+    const int rc = timed_launch(b, 0, [&]() -> int {
+        CU(launch(srd));
+        return OPN_OK;
+    });
+    if (rc) return rc;
+    CU(cudaEventRecord(b->ev_rd[p], srd));
+    b->launches[0]++;
+    return OPN_OK;
+}
+
+// streams [group_first(n, g, G), group_first(n, g + 1, G)) of n are group g of G
+uint32_t group_first(uint32_t n, int g, int G) { return (uint32_t)((uint64_t)n * (uint32_t)g / (uint32_t)G); }
+
+// The number of launches a step's frame kernel is cut into.  A device-resident step (item k = stream k) of a large batch
+// runs as NGROUPS launches, group g over items [group_first(n, g, G), group_first(n, g + 1, G)); a host-path bucket (any
+// subset of the streams, in any order) runs as one.
+int frame_groups(const opn_batch *b, bool device_step)
+{
+    return device_step && b->n >= opn_batch::GROUP_MIN_ITEMS ? opn_batch::NGROUPS : 1;
+}
+
+// The frame kernel of a step on buffer set p, after its range decode: launch(g, st) enqueues group g of G on st.  One group
+// runs on `stream` after whatever the other groups' streams hold.  G groups: group 0 on `stream`, the others on their
+// own streams, each after its own previous frames (stream order), this step's range decode and whatever `stream` held
+// when the groups were last joined.  A timed pass joins them again before its end event.
+template <class F> int frame_launches(opn_batch *b, int p, int G, F &&launch)
+{
+    const int rc = timed_launch(b, 1, [&]() -> int {
+        if (G == 1) {
+            const int rc = join_groups(b);  // streams of the other groups' ranges may be in this bucket
+            if (rc) return rc;
+            CU(cudaStreamWaitEvent(b->stream, b->ev_rd[p], 0));
+            CU(launch(0, b->stream));
+            b->launches[1]++;
+            return OPN_OK;
+        }
+        CU(cudaEventRecord(b->ev_sw, b->stream));
+        for (int g = 0; g < G; g++) {
+            const cudaStream_t st = g == 0 ? b->stream : b->stream_fr[g];
+            if (g > 0 && !b->fr_pending[g]) CU(cudaStreamWaitEvent(st, b->ev_sw, 0));
+            CU(cudaStreamWaitEvent(st, b->ev_rd[p], 0));
+            CU(launch(g, st));
+            b->launches[1]++;
+            if (g > 0) {
+                CU(cudaEventRecord(b->ev_fr[p][g], st));
+                b->fr_pending[g] = true;
+                b->fr_last_set[g] = p;
+            }
+        }
+        return b->timing ? join_groups(b) : OPN_OK;
+    });
+    if (rc) return rc;
+    CU(cudaEventRecord(b->ev_k1[p], b->stream));
+    b->k1_recorded[p] = true;
+    b->k1_grouped[p] = G > 1;
+    return OPN_OK;
+}
+
+// One bucket = items of equal frame size that may run concurrently.
 // softclip_reset: a float call clears the soft-clip memory of every stream that decodes a packet (decoder.rs:420-423).
 int run_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, const uint32_t *d_lens,
                const uint32_t *d_stream_idx, const uint32_t *d_dense_off, uint32_t n_items, int lm, int has_toc,
@@ -358,10 +404,8 @@ int run_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, 
 {
     Range nv("opn: step (range decode + frame kernel)");
     if (stream_channels == 0) stream_channels = b->cfg.channels;
-    if (stream_channels != b->cfg.channels && b->unfused) return OPN_ERR_UNIMPLEMENTED;  // the measurement variant maps nothing
-    const int p = b->set;
-    b->set = (p + 1) % opn_batch::NSETS;
-    cudaStream_t srd = b->stream_rd[p % opn_batch::NRD];
+    const int p = begin_step(b, false, inputs_on);
+    if (p < 0) return p;
     SymbolArgs s{};
     s.arena = d_arena;
     s.offsets = d_offsets;
@@ -371,58 +415,16 @@ int run_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, 
     s.lm = lm;
     s.channels = stream_channels;  // the range decode follows the packets' layout
     s.has_toc = has_toc;
-    s.side = nullptr;
     s.hdr = b->d_hdr[p];
     s.status = b->d_status[p];
-    s.coef = b->unfused ? b->d_coef[p] : nullptr;
-    s.y_out = nullptr;
     s.idx = b->d_idx[p];
     s.pkt_cap = pkt_cap;
     s.parts = b->d_parts[p];
     s.bande = b->d_bande[p];
-    s.side2 = nullptr;
     const bool celt2 = b->cfg.bitstream == OPN_BITSTREAM_SYNTH_CELT_2;
-    int rc;
-    if (b->timing) {
-        // measurement pass: everything in order on one stream, events around each stage
-        if (inputs_on == 2) {
-            CU(cudaEventRecord(b->ev_in, b->stream_up));
-            CU(cudaStreamWaitEvent(b->stream, b->ev_in, 0));
-        }
-        rc = timed_launch(b, 0, do_rangedec, &s);
-        if (rc) return rc;
-        if (b->unfused) {
-            rc = timed_launch(b, 2, do_expand, &s);
-            if (rc) return rc;
-        }
-    } else {
-        if (inputs_on == 1) {
-            CU(cudaEventRecord(b->ev_in, b->stream));
-            CU(cudaStreamWaitEvent(srd, b->ev_in, 0));
-        } else if (inputs_on == 2) {
-            CU(cudaEventRecord(b->ev_in, b->stream_up));
-            CU(cudaStreamWaitEvent(srd, b->ev_in, 0));
-        }
-        if (b->k1_recorded[p]) {  // set p is free again
-            CU(cudaStreamWaitEvent(srd, b->ev_k1[p], 0));
-            if (b->k1_grouped[p])
-                for (int g = 1; g < opn_batch::NGROUPS; g++) CU(cudaStreamWaitEvent(srd, b->ev_fr[p][g], 0));
-        }
-        CU(celt2 ? launch_celt2_rangedec(s, srd) : launch_synth_rangedec(s, srd));
-        CU(cudaEventRecord(b->ev_rd[p], srd));
-        b->launches[0]++;
-        if (b->unfused) {
-            CU(cudaStreamWaitEvent(b->stream_ex, b->ev_rd[p], 0));
-            CU(launch_synth_expand(s, b->stream_ex));
-            CU(cudaEventRecord(b->ev_ex[p], b->stream_ex));
-            CU(cudaStreamWaitEvent(b->stream, b->ev_ex[p], 0));
-            b->launches[2]++;
-        } else {
-            CU(cudaStreamWaitEvent(b->stream, b->ev_rd[p], 0));
-        }
-    }
+    int rc = range_decode(b, p, [&](cudaStream_t st) { return celt2 ? launch_celt2_rangedec(s, st) : launch_synth_rangedec(s, st); });
+    if (rc) return rc;
     FrameArgs m{};
-    m.coef = b->unfused ? b->d_coef[p] : nullptr;
     m.idx = celt2 ? nullptr : b->d_idx[p];
     m.parts = celt2 ? b->d_parts[p] : nullptr;
     m.bande = b->d_bande[p];
@@ -431,8 +433,6 @@ int run_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, 
     m.stream_idx = d_stream_idx;
     m.dense_off = d_dense_off;
     m.n_items = n_items;
-    m.item0 = 0;
-    m.item_end = n_items;
     m.lm = lm;
     m.channels = b->cfg.channels;
     m.stream_channels = stream_channels;
@@ -448,47 +448,13 @@ int run_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, 
     m.final_range = b->d_final;
     m.softclip_reset = softclip_reset ? b->d_softclip : nullptr;
     m.hist_samples = b->timing ? b->d_hist_samples : nullptr;
-    const bool grouped = !b->timing && frame_grouped(b, m);
-    if (b->timing) {
-        rc = join_groups(b);
-        if (rc) return rc;
-        rc = timed_launch(b, 1, do_frame, &m);
-        if (rc) return rc;
-        if (frame_grouped(b, m)) b->launches[1] += opn_batch::NGROUPS - 1;
-    } else if (!grouped) {
-        rc = join_groups(b);  // streams of the other groups' ranges may be in this bucket
-        if (rc) return rc;
-        CU(launch_frame(m, b->stream));
-        b->launches[1]++;
-    } else {
-        // group 0 on `stream`, the others on their own streams: each after its own previous frames (stream order), after
-        // this step's range decode and after whatever `stream` held when the groups were last joined
-        CU(cudaEventRecord(b->ev_sw, b->stream));
-        for (int g = 0; g < opn_batch::NGROUPS; g++) {
-            cudaStream_t st = g == 0 ? b->stream : b->stream_fr[g];
-            if (g > 0) {
-                if (!b->fr_pending[g]) CU(cudaStreamWaitEvent(st, b->ev_sw, 0));
-                CU(cudaStreamWaitEvent(st, b->ev_rd[p], 0));
-            }
-            m.item0 = (uint32_t)((uint64_t)n_items * g / opn_batch::NGROUPS);
-            m.item_end = (uint32_t)((uint64_t)n_items * (g + 1) / opn_batch::NGROUPS);
-            CU(launch_frame(m, st));
-            b->launches[1]++;
-            if (g > 0) {
-                CU(cudaEventRecord(b->ev_fr[p][g], st));
-                b->fr_pending[g] = true;
-                b->fr_last_set[g] = p;
-            }
-        }
-    }
-    CU(cudaEventRecord(b->ev_k1[p], b->stream));
-    b->k1_recorded[p] = true;
-    b->k1_grouped[p] = grouped;
-    return OPN_OK;
+    const int G = frame_groups(b, !d_stream_idx);
+    return frame_launches(b, p, G, [&](int g, cudaStream_t st) {
+        m.item0 = group_first(n_items, g, G);
+        m.item_end = group_first(n_items, g + 1, G);
+        return launch_frame(m, st);
+    });
 }
-
-cudaError_t do_silk_rangedec(opn_batch *b, const void *a) { return launch_silk_rangedec(*static_cast<const SilkArgs *>(a), b->stream); }
-cudaError_t do_silk_frame(opn_batch *b, const void *a) { return launch_silk_frame(*static_cast<const SilkArgs *>(a), b->stream); }
 
 // One bucket of SILK-only frames (SYNTH-SILK/1) of one duration and one coded channel count: the range decode on an entropy
 // stream (it may run ahead like the CELT one), the frame kernel on the batch stream (it owns the streams' filter state and
@@ -499,9 +465,8 @@ int run_silk_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offs
 {
     Range nv("opn: SILK step (range decode + frame kernel)");
     if (!b->silk) return OPN_ERR_UNIMPLEMENTED;  // silk/decoder.rs:79
-    const int p = b->set;
-    b->set = (p + 1) % opn_batch::NSETS;
-    cudaStream_t srd = b->stream_rd[p % opn_batch::NRD];
+    const int p = begin_step(b, false, inputs_on);
+    if (p < 0) return p;
     SilkArgs a{};
     a.arena = d_arena;
     a.offsets = d_offsets;
@@ -527,65 +492,16 @@ int run_silk_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offs
     a.result = d_result;
     a.final_range = b->d_final;
     a.softclip_reset = softclip_reset ? b->d_softclip : nullptr;
-    // a large device-resident bucket (item k = stream k) runs as NGROUPS concurrent launches, group g on the stream that owns
-    // streams [n g / G, n (g+1) / G) -- the same cut as the CELT frame kernel's, so a stream's frames stay in order whatever it sends
-    const bool grouped = !b->timing && opn_batch::NGROUPS > 1 && !d_stream_idx && n_items == b->n && n_items >= opn_batch::GROUP_MIN_ITEMS;
-    int rc = OPN_OK;
-    if (!grouped) rc = join_groups(b);  // frame kernels of these streams may still run on the group streams
+    int rc = range_decode(b, p, [&](cudaStream_t st) { return launch_silk_rangedec(a, st); });
     if (rc) return rc;
-    if (b->timing) {
-        if (inputs_on == 2) {
-            CU(cudaEventRecord(b->ev_in, b->stream_up));
-            CU(cudaStreamWaitEvent(b->stream, b->ev_in, 0));
-        }
-        rc = timed_launch(b, 0, do_silk_rangedec, &a);
-        if (rc) return rc;
-        rc = timed_launch(b, 1, do_silk_frame, &a);
-        if (rc) return rc;
-    } else {
-        if (inputs_on == 1) {
-            CU(cudaEventRecord(b->ev_in, b->stream));
-            CU(cudaStreamWaitEvent(srd, b->ev_in, 0));
-        } else if (inputs_on == 2) {
-            CU(cudaEventRecord(b->ev_in, b->stream_up));
-            CU(cudaStreamWaitEvent(srd, b->ev_in, 0));
-        }
-        if (b->k1_recorded[p]) {  // set p is free again
-            CU(cudaStreamWaitEvent(srd, b->ev_k1[p], 0));
-            if (b->k1_grouped[p])
-                for (int g = 1; g < opn_batch::NGROUPS; g++) CU(cudaStreamWaitEvent(srd, b->ev_fr[p][g], 0));
-        }
-        CU(launch_silk_rangedec(a, srd));
-        CU(cudaEventRecord(b->ev_rd[p], srd));
-        b->launches[0]++;
-        if (!grouped) {
-            CU(cudaStreamWaitEvent(b->stream, b->ev_rd[p], 0));
-            CU(launch_silk_frame(a, b->stream));
-            b->launches[1]++;
-        } else {
-            // like the CELT frame kernel: contiguous thirds of the streams on three CUDA streams, each after its own previous
-            // frames.  The serial LPC phase of one group's CTAs then overlaps the parallel phases of the others'.
-            CU(cudaEventRecord(b->ev_sw, b->stream));
-            for (int g = 0; g < opn_batch::NGROUPS; g++) {
-                cudaStream_t st = g == 0 ? b->stream : b->stream_fr[g];
-                if (g > 0 && !b->fr_pending[g]) CU(cudaStreamWaitEvent(st, b->ev_sw, 0));
-                CU(cudaStreamWaitEvent(st, b->ev_rd[p], 0));
-                a.item0 = group_first(n_items, g, opn_batch::NGROUPS);
-                a.item_end = group_first(n_items, g + 1, opn_batch::NGROUPS);
-                CU(launch_silk_frame(a, st));
-                b->launches[1]++;
-                if (g > 0) {
-                    CU(cudaEventRecord(b->ev_fr[p][g], st));
-                    b->fr_pending[g] = true;
-                    b->fr_last_set[g] = p;
-                }
-            }
-        }
-    }
-    CU(cudaEventRecord(b->ev_k1[p], b->stream));
-    b->k1_recorded[p] = true;
-    b->k1_grouped[p] = grouped;
-    return OPN_OK;
+    // Groups as for the CELT frame kernel: the serial LPC phase of one group's CTAs then overlaps the parallel phases of the
+    // others'.  A timed pass launches the SILK frame kernel once.
+    const int G = b->timing ? 1 : frame_groups(b, !d_stream_idx);
+    return frame_launches(b, p, G, [&](int g, cudaStream_t st) {
+        a.item0 = group_first(n_items, g, G);
+        a.item_end = group_first(n_items, g + 1, G);
+        return launch_silk_frame(a, st);
+    });
 }
 
 int mix_alloc(opn_batch *b)
@@ -602,7 +518,8 @@ int mix_alloc(opn_batch *b)
     }
     uint8_t *p = nullptr;
     CU(cudaMalloc(&p, n));
-    CU(cudaMemsetAsync(p, MIX_NO_ITEM, n, b->stream_ex));
+    CU(cudaMemsetAsync(p, MIX_NO_ITEM, n, b->stream_mix));
+    CU(cudaStreamSynchronize(b->stream_mix));  // a timed pass buckets on `stream`
     b->d_last_lm = p;
     return OPN_OK;
 }
@@ -613,15 +530,13 @@ int mix_alloc(opn_batch *b)
 int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, const uint32_t *d_lens, size_t capacity, float *dense,
               size_t dense_stride, int32_t *d_result, int inputs_on, bool softclip_reset)
 {
-    if (b->unfused) return OPN_ERR_UNIMPLEMENTED;  // the measurement variant has no mixed-frame kernel
     Range nv("opn: mixed-frame step (bucketing + range decode + frame kernel)");
     int rc = mix_alloc(b);
     if (rc) return rc;
-    const int p = b->set;
-    b->set = (p + 1) % opn_batch::NSETS;
-    cudaStream_t srd = b->stream_rd[p % opn_batch::NRD];
+    const int p = begin_step(b, true, inputs_on);
+    if (p < 0) return p;
     const uint32_t cap = mix_item_cap(b->n);
-    const int G = mix_groups(b);
+    const int G = frame_groups(b, true);
     MixArgs x{};
     x.arena = d_arena;
     x.offsets = d_offsets;
@@ -678,63 +593,16 @@ int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, c
     m.softclip_reset = softclip_reset ? b->d_softclip : nullptr;
     m.hist_samples = b->timing ? b->d_hist_samples : nullptr;
     m.plan = b->d_mix_plan[p];
-    if (b->timing) {
-        // measurement pass: everything in order on `stream`
-        rc = join_groups(b);
-        if (rc) return rc;
-        CU(cudaStreamSynchronize(b->stream_ex));  // earlier steps' bucketing (it owns last_lm)
-        CU(launch_mix_plan(x, b->stream));
-        b->launches[2] += 2;
-        rc = timed_launch(b, 0, do_rangedec, &s);
-        if (rc) return rc;
-        rc = timed_launch(b, 1, do_frame, &m);
-        if (rc) return rc;
-        b->launches[1] += G - 1;
-    } else {
-        cudaStream_t sx = b->stream_ex;
-        if (inputs_on == 1) {
-            CU(cudaEventRecord(b->ev_in, b->stream));
-            CU(cudaStreamWaitEvent(sx, b->ev_in, 0));
-        }
-        if (b->k1_recorded[p]) {  // set p (its item table and plan included) is free again
-            CU(cudaStreamWaitEvent(sx, b->ev_k1[p], 0));
-            if (b->k1_grouped[p])
-                for (int g = 1; g < opn_batch::NGROUPS; g++) CU(cudaStreamWaitEvent(sx, b->ev_fr[p][g], 0));
-        }
-        CU(launch_mix_plan(x, sx));
-        b->launches[2] += 2;
-        CU(cudaEventRecord(b->ev_mix[p], sx));
-        CU(cudaStreamWaitEvent(srd, b->ev_mix[p], 0));
-        CU(celt2 ? launch_celt2_rangedec(s, srd) : launch_synth_rangedec(s, srd));
-        CU(cudaEventRecord(b->ev_rd[p], srd));
-        b->launches[0]++;
-        if (G == 1) {
-            rc = join_groups(b);
-            if (rc) return rc;
-            CU(cudaStreamWaitEvent(b->stream, b->ev_rd[p], 0));
-            CU(launch_frame_mix(m, b->n, b->stream));
-            b->launches[1]++;
-        } else {
-            CU(cudaEventRecord(b->ev_sw, b->stream));
-            for (int g = 0; g < G; g++) {
-                cudaStream_t st = g == 0 ? b->stream : b->stream_fr[g];
-                if (g > 0 && !b->fr_pending[g]) CU(cudaStreamWaitEvent(st, b->ev_sw, 0));
-                CU(cudaStreamWaitEvent(st, b->ev_rd[p], 0));
-                m.group = g;
-                CU(launch_frame_mix(m, group_first(b->n, g + 1, G) - group_first(b->n, g, G), st));
-                b->launches[1]++;
-                if (g > 0) {
-                    CU(cudaEventRecord(b->ev_fr[p][g], st));
-                    b->fr_pending[g] = true;
-                    b->fr_last_set[g] = p;
-                }
-            }
-        }
-    }
-    CU(cudaEventRecord(b->ev_k1[p], b->stream));
-    b->k1_recorded[p] = true;
-    b->k1_grouped[p] = !b->timing && G > 1;
-    return OPN_OK;
+    CU(launch_mix_plan(x, mix_stream(b)));
+    b->launches[2] += 2;
+    rc = order_after(b->ev_mix[p], mix_stream(b), rd_stream(b, p));
+    if (rc) return rc;
+    rc = range_decode(b, p, [&](cudaStream_t st) { return celt2 ? launch_celt2_rangedec(s, st) : launch_synth_rangedec(s, st); });
+    if (rc) return rc;
+    return frame_launches(b, p, G, [&](int g, cudaStream_t st) {
+        m.group = g;
+        return launch_frame_mix(m, group_first(b->n, g + 1, G) - group_first(b->n, g, G), st);
+    });
 }
 
 // PLC sizing of decode_native(None)/decode_frame(None), src/decoder.rs:427-441 and 467-513.
@@ -840,8 +708,6 @@ int opn_batch_create(int device, uint32_t n_streams, const opn_config *cfg, opn_
     b->cfg.bitstream = celt_bitstream;  // how CELT frames are laid out; the SILK opt-in is b->silk
     b->silk = (cfg->bitstream & OPN_BITSTREAM_SYNTH_SILK_1) != 0;
     b->gain = host_gain_from_q8(cfg->gain_q8);
-    const char *uf = std::getenv("OPN_UNFUSED_EXPAND");
-    b->unfused = uf && uf[0] == '1' && celt_bitstream == OPN_BITSTREAM_SYNTH_CELT_1;
     const size_t n = n_streams, C = (size_t)cfg->channels;
     cudaError_t e = cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking);
     // All pipeline streams have the same priority (measured in round 1, tools/experiments/priorities.sh: raising the
@@ -851,9 +717,8 @@ int opn_batch_create(int device, uint32_t n_streams, const opn_config *cfg, opn_
         // the highest priority, so that its CTAs are placed first whenever a frame-kernel CTA retires (125 -> 116 us per
         // step).  SYNTH-CELT/1: no difference in steady state (44.3 us either way), but a short burst loses 2-3 us per step
         // (20 steps after a drained pipeline: 47.9-49.2 us at equal priority, 50.2-52.5 with the range decodes of eight
-        // steps placed ahead of the first frame kernels), so those keep the default.  OPN_RD_PRIORITY=0/1 overrides.
-        const char *pr = std::getenv("OPN_RD_PRIORITY");
-        const bool high = pr ? pr[0] == '1' : celt_bitstream == OPN_BITSTREAM_SYNTH_CELT_2;
+        // steps placed ahead of the first frame kernels), so those keep the default.
+        const bool high = celt_bitstream == OPN_BITSTREAM_SYNTH_CELT_2;
         int lo_p = 0, hi_p = 0;
         if (high) cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p);
         for (int q = 0; q < opn_batch::NRD && e == cudaSuccess; q++)
@@ -861,21 +726,18 @@ int opn_batch_create(int device, uint32_t n_streams, const opn_config *cfg, opn_
     }
     for (int q = 0; q < opn_batch::NSETS && e == cudaSuccess; q++) {
         e = cudaEventCreateWithFlags(&b->ev_rd[q], cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->ev_ex[q], cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->ev_k1[q], cudaEventDisableTiming);
         for (int g = 1; g < opn_batch::NGROUPS && e == cudaSuccess; g++) e = cudaEventCreateWithFlags(&b->ev_fr[q][g], cudaEventDisableTiming);
         if (e == cudaSuccess) e = cudaMalloc(&b->d_idx[q], n * 72 * sizeof(uint32_t));
-        if (e == cudaSuccess && b->unfused) e = cudaMalloc(&b->d_coef[q], n * C * 960 * sizeof(float));
         if (e == cudaSuccess) e = cudaMalloc(&b->d_hdr[q], n * sizeof(uint4));
         if (e == cudaSuccess && celt_bitstream == OPN_BITSTREAM_SYNTH_CELT_2) e = cudaMalloc(&b->d_parts[q], n * CELT2_MAX_PARTS * sizeof(Celt2Part));
         if (e == cudaSuccess && b->silk) e = cudaMalloc(&b->d_silk_rec[q], n * 2 * sizeof(SilkRec));
         if (e == cudaSuccess && celt_bitstream == OPN_BITSTREAM_SYNTH_CELT_2) e = cudaMalloc(&b->d_bande[q], n * 42 * sizeof(int16_t));
         if (e == cudaSuccess) e = cudaMalloc(&b->d_status[q], n * sizeof(int32_t));
     }
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&b->stream_ex, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&b->stream_mix, cudaStreamNonBlocking);
     for (int g = 1; g < opn_batch::NGROUPS && e == cudaSuccess; g++) e = cudaStreamCreateWithFlags(&b->stream_fr[g], cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->ev_sw, cudaEventDisableTiming);
-    for (int g = 1; g < opn_batch::NGROUPS && e == cudaSuccess; g++) e = cudaEventCreateWithFlags(&b->ev_tm[g], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->ev_in, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&b->stream_up, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&b->stream_dn, cudaStreamNonBlocking);
@@ -920,7 +782,7 @@ void opn_batch_destroy(opn_batch *b)
     cudaSetDevice(b->device);
     for (int q = 0; q < opn_batch::NRD; q++)
         if (b->stream_rd[q]) cudaStreamSynchronize(b->stream_rd[q]);
-    for (cudaStream_t st : {b->stream_ex, b->stream_up, b->stream, b->stream_dn})
+    for (cudaStream_t st : {b->stream_mix, b->stream_up, b->stream, b->stream_dn})
         if (st) cudaStreamSynchronize(st);
     for (int g = 1; g < opn_batch::NGROUPS; g++)
         if (b->stream_fr[g]) {
@@ -928,16 +790,12 @@ void opn_batch_destroy(opn_batch *b)
             cudaStreamDestroy(b->stream_fr[g]);
         }
     if (b->ev_sw) cudaEventDestroy(b->ev_sw);
-    for (int g = 1; g < opn_batch::NGROUPS; g++)
-        if (b->ev_tm[g]) cudaEventDestroy(b->ev_tm[g]);
     for (int q = 0; q < opn_batch::NSETS; q++) {
         for (int g = 1; g < opn_batch::NGROUPS; g++)
             if (b->ev_fr[q][g]) cudaEventDestroy(b->ev_fr[q][g]);
         if (b->ev_rd[q]) cudaEventDestroy(b->ev_rd[q]);
-        if (b->ev_ex[q]) cudaEventDestroy(b->ev_ex[q]);
         if (b->ev_k1[q]) cudaEventDestroy(b->ev_k1[q]);
         cudaFree(b->d_idx[q]);
-        cudaFree(b->d_coef[q]);
         cudaFree(b->d_hdr[q]);
         cudaFree(b->d_parts[q]);
         cudaFree(b->d_bande[q]);
@@ -953,7 +811,7 @@ void opn_batch_destroy(opn_batch *b)
     if (b->ev_in) cudaEventDestroy(b->ev_in);
     for (int q = 0; q < opn_batch::MAX_CHUNKS; q++)
         if (b->ev_chunk[q]) cudaEventDestroy(b->ev_chunk[q]);
-    for (cudaStream_t st : {b->stream_ex, b->stream_up, b->stream_dn})
+    for (cudaStream_t st : {b->stream_mix, b->stream_up, b->stream_dn})
         if (st) cudaStreamDestroy(st);
     for (int q = 0; q < opn_batch::NRD; q++)
         if (b->stream_rd[q]) cudaStreamDestroy(b->stream_rd[q]);

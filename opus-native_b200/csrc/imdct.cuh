@@ -16,7 +16,7 @@ namespace opn {
 // recovers from the way the operand is put together here (p_add(a, make_float2(s.y, -s.x)) is ONE FADD2).
 // Only sums are packed.  ptxas contracts mul.rn.f32x2 followed by add.rn.f32x2 into FFMA2 even under --fmad=false
 // (checked on 12.9), which would change roundings; a scalar FMUL is never contracted, so every product that feeds a sum
-// stays scalar.  tests/test_host_logic.py::test_no_fma_in_the_float_kernels looks at the SASS.
+// stays scalar.  tests/test_host_logic.py::test_no_fma_in_the_fused_float_kernels looks at the SASS.
 __device__ __forceinline__ float2 p_add(float2 a, float2 b)
 {
     float2 r;

@@ -83,7 +83,6 @@ struct SymbolArgs {
 };
 
 struct FrameArgs {
-    const float *coef;            // [n_streams][C][120<<lm] coefficient rows (unfused variant only)
     const uint32_t *idx;          // [n_streams][72] PVQ codeword indices (range decode output, SYNTH-CELT/1)
     const struct Celt2Part *parts;  // [n_streams][CELT2_MAX_PARTS] PVQ leaves (range decode output, SYNTH-CELT/2) or nullptr
     const uint4 *hdr;             // [n_streams] frame headers (range decode output)
@@ -194,7 +193,7 @@ cudaError_t launch_synth_rangedec(const SymbolArgs &a, cudaStream_t st);  // sta
 cudaError_t launch_synth_expand(const SymbolArgs &a, cudaStream_t st);    // stage 0b: one warp per packet
 cudaError_t launch_celt2_rangedec(const SymbolArgs &a, cudaStream_t st);  // SYNTH-CELT/2: one lane per packet -> header + part list
 cudaError_t launch_celt2_expand(const SymbolArgs &a, cudaStream_t st);    // SYNTH-CELT/2 operator: part lists -> coefficient rows
-// the frame kernel: (PVQ expansion when a.coef == nullptr) + IMDCT + TDAC + comb post-filter + PCM store
+// the frame kernel: PVQ expansion + IMDCT + TDAC + comb post-filter + PCM store
 cudaError_t launch_frame(const FrameArgs &a, cudaStream_t st);
 // mixed-frame step: bucketing (two kernels on one stream) and the frame kernel of one group (a.plan, a.group; grid sized by the
 // caller's upper bound n_streams_in_group)

@@ -32,8 +32,6 @@ template <int LM, int C> static cudaError_t set_carveout()
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_frame_w<LM, C, FRAME_SYNTH1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_frame_w<LM, C, FRAME_SYNTH2>, cudaFuncAttributePreferredSharedMemoryCarveout, W_CARVEOUT_PCT);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_frame_w<LM, C, FRAME_SYNTH2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_frame_w<LM, C, FRAME_ROWS>, cudaFuncAttributePreferredSharedMemoryCarveout, W_CARVEOUT_PCT);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_frame_w<LM, C, FRAME_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     return e;
 }
 template <int LM, int C, int CS> static cudaError_t set_carveout_cross()
@@ -323,8 +321,7 @@ template <int LM, int C> static cudaError_t launch_frame_w(const FrameArgs &a, c
 {
     const size_t smem = frame_smem_bytes(LM, C, g_fblob_bytes[LM][C - 1]);
     const uint32_t grid = (a.item_end - a.item0 + FRAME_WARPS - 1) / FRAME_WARPS;
-    if (a.coef) k_frame_w<LM, C, FRAME_ROWS><<<grid, 32 * FRAME_WARPS, smem, st>>>(a);
-    else if (a.parts) k_frame_w<LM, C, FRAME_SYNTH2><<<grid, 32 * FRAME_WARPS, smem, st>>>(a);
+    if (a.parts) k_frame_w<LM, C, FRAME_SYNTH2><<<grid, 32 * FRAME_WARPS, smem, st>>>(a);
     else k_frame_w<LM, C, FRAME_SYNTH1><<<grid, 32 * FRAME_WARPS, smem, st>>>(a);
     return cudaGetLastError();
 }
@@ -332,7 +329,6 @@ template <int LM, int C> static cudaError_t launch_frame_w(const FrameArgs &a, c
 // packets of CS channels into a decoder of C != CS channels (mono <-> stereo mapping inside the frame kernel)
 template <int LM, int C, int CS> static cudaError_t launch_frame_cross(const FrameArgs &a, cudaStream_t st)
 {
-    if (a.coef) return cudaErrorInvalidValue;
     const size_t smem = frame_smem_bytes(LM, 2, g_fblob_bytes[LM][CS - 1]);
     const uint32_t grid = (a.item_end - a.item0 + FRAME_WARPS - 1) / FRAME_WARPS;
     if (a.parts) k_frame_w<LM, C, FRAME_SYNTH2, CS><<<grid, 32 * FRAME_WARPS, smem, st>>>(a);
@@ -399,7 +395,7 @@ cudaError_t launch_synth_symbols(const SymbolArgs &a, cudaStream_t st)
 cudaError_t launch_frame(const FrameArgs &a, cudaStream_t st)
 {
     if (a.item_end <= a.item0) return cudaSuccess;
-    if (!a.coef && !a.idx && !a.parts) return cudaErrorInvalidValue;
+    if (!a.idx && !a.parts) return cudaErrorInvalidValue;
     if (a.stream_channels != 0 && a.stream_channels != a.channels) {
         switch (a.lm * 2 + (a.channels - 1)) {
         case 0: return launch_frame_cross<0, 1, 2>(a, st);
@@ -445,7 +441,7 @@ cudaError_t launch_mix_plan(const MixArgs &a, cudaStream_t st)
 cudaError_t launch_frame_mix(const FrameArgs &a, uint32_t n_streams_in_group, cudaStream_t st)
 {
     if (n_streams_in_group == 0) return cudaSuccess;
-    if (!a.plan || a.group < 0 || a.group >= MIX_GROUPS || a.coef || (!a.idx && !a.parts) || !a.stream_idx) return cudaErrorInvalidValue;
+    if (!a.plan || a.group < 0 || a.group >= MIX_GROUPS || (!a.idx && !a.parts) || !a.stream_idx) return cudaErrorInvalidValue;
     const uint32_t grid = (n_streams_in_group + FRAME_WARPS - 1) / FRAME_WARPS + 4u;  // each of the four buckets rounds up
     const size_t smem = mix_smem_bytes(a.channels);
     if (a.channels == 2) {

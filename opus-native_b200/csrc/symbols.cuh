@@ -495,8 +495,8 @@ __device__ __forceinline__ void w_expand(const ExpandTables &T, int lm, uint32_t
     }
 }
 
-// Stand-alone expansion kernel (operator entry opn_op_synth_symbols and the unfused pipeline variant): the same w_expand
-// the frame kernel runs, with the PVQ tables staged in shared memory by TMA; the coefficient rows leave as float4.
+// Stand-alone expansion kernel (operator entry opn_op_synth_symbols): the same w_expand the frame kernel runs, with the PVQ
+// tables staged in shared memory by TMA; the coefficient rows leave as float4.
 __global__ void __launch_bounds__(EXPAND_WARPS_PER_CTA * 32) k_synth_expand(SymbolArgs A)
 {
     extern __shared__ __align__(16) uint8_t smem[];
