@@ -360,7 +360,7 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
         old.period = (int32_t)q.x;
         old.tapset = (int32_t)q.y;
         old.gain = __uint_as_float(q.z);
-        old.pad = 0;
+        old.lm1 = (int32_t)q.w;
     }
     const uint32_t pos = stash[2].x;
     const int s_on = (hdr.x >> 1) & 1u, s_tapset = (hdr.x >> 4) & 15u, s_gain = (hdr.x >> 8) & 15u, s_period = hdr.x >> 16;
@@ -419,7 +419,7 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
         nw.period = t1;
         nw.tapset = tap1;
         nw.gain = g1;
-        nw.pad = 0;
+        nw.lm1 = lost ? old.lm1 : LM + 1;  // the frame size a mixed-frame step conceals a lost packet with (k_mix_key)
         A.pf[stream] = nw;
         if (A.result) A.result[stream] = NF;
         if (A.final_range) A.final_range[stream] = lost ? 0u : hdr.y;
@@ -463,6 +463,10 @@ __global__ void __launch_bounds__(256) k_mix_key(MixArgs A)
     uint32_t key = MIX_NO_ITEM;
     int32_t err = 0;
     if (on) {
+        if (A.pf) {  // after other CELT steps (their frame kernels have finished): they recorded each stream's last frame size
+            const int32_t l1 = A.pf[s].lm1;
+            A.last_lm[s] = l1 > 0 ? (uint8_t)(l1 - 1) : (uint8_t)MIX_NO_ITEM;
+        }
         const uint32_t len = A.lens[s];
         int lm = -1;
         if (len == 0u) {

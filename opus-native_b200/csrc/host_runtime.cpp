@@ -186,6 +186,12 @@ struct opn_batch {
     // mixed-frame steps (OPN_FLAG_MIXED_FRAMES), allocated on first use: the step's buckets are built on the device
     // (k_mix_key / k_mix_place on stream_mix, in step order) into one item table + plan per buffer set
     uint8_t *d_last_lm = nullptr, *d_mix_key = nullptr;  // [n] state: LM of the last decoded packet; scratch: bucket of the stream
+    // A lost packet of a mixed-frame step conceals one frame of the size of the stream's last decoded frame, whichever kind
+    // of step decoded it.  k_mix_key keeps d_last_lm for mixed-frame steps; every CELT frame kernel also records the size in
+    // the stream's PfState::lm1.  Bucketing runs ahead of the frame kernels on stream_mix, so a mixed-frame step that follows
+    // other CELT steps first waits for their frame kernels and then takes d_last_lm from PfState::lm1.
+    bool lm_pending = false;  // CELT steps other than mixed-frame ones ran since the last mixed-frame step's bucketing
+    int lm_set = 0;
     uint32_t *d_mix_rank = nullptr;                      // [n] scratch
     uint32_t *d_mix_items[NSETS] = {};                   // [3][mix_item_cap(n)]: offsets | lens | stream ids, by item
     uint8_t *d_mix_lm[NSETS] = {};                       // [mix_item_cap(n)]
@@ -449,11 +455,15 @@ int run_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, 
     m.softclip_reset = softclip_reset ? b->d_softclip : nullptr;
     m.hist_samples = b->timing ? b->d_hist_samples : nullptr;
     const int G = frame_groups(b, !d_stream_idx);
-    return frame_launches(b, p, G, [&](int g, cudaStream_t st) {
+    rc = frame_launches(b, p, G, [&](int g, cudaStream_t st) {
         m.item0 = group_first(n_items, g, G);
         m.item_end = group_first(n_items, g + 1, G);
         return launch_frame(m, st);
     });
+    if (rc) return rc;
+    b->lm_pending = true;
+    b->lm_set = p;
+    return OPN_OK;
 }
 
 // One bucket of SILK-only frames (SYNTH-SILK/1) of one duration and one coded channel count: the range decode on an entropy
@@ -593,6 +603,15 @@ int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, c
     m.softclip_reset = softclip_reset ? b->d_softclip : nullptr;
     m.hist_samples = b->timing ? b->d_hist_samples : nullptr;
     m.plan = b->d_mix_plan[p];
+    x.pf = nullptr;
+    if (b->lm_pending) {  // k_mix_key takes the frame sizes from the post-filter state, after the other steps' frame kernels
+        const int q = b->lm_set;
+        CU(cudaStreamWaitEvent(mix_stream(b), b->ev_k1[q], 0));
+        if (b->k1_grouped[q])
+            for (int g = 1; g < opn_batch::NGROUPS; g++) CU(cudaStreamWaitEvent(mix_stream(b), b->ev_fr[q][g], 0));
+        x.pf = b->d_pf;
+        b->lm_pending = false;
+    }
     CU(launch_mix_plan(x, mix_stream(b)));
     b->launches[2] += 2;
     rc = order_after(b->ev_mix[p], mix_stream(b), rd_stream(b, p));
@@ -871,6 +890,7 @@ int opn_batch_reset(opn_batch *b)  // DecoderInner::reset, decoder.rs:286-303, f
     b->set = 0;
     CU(cudaMemsetAsync(b->d_softclip, 0, n * 2 * sizeof(float), b->stream));
     if (b->d_last_lm) CU(cudaMemsetAsync(b->d_last_lm, MIX_NO_ITEM, n, b->stream));
+    b->lm_pending = false;
     if (b->silk) {
         CU(cudaMemsetAsync(b->d_silk.slpc, 0, n * 2 * 16 * sizeof(int32_t), b->stream));
         CU(cudaMemsetAsync(b->d_silk.hist, 0, n * 2 * SILK_HIST * sizeof(int32_t), b->stream));

@@ -31,7 +31,7 @@ constexpr int32_t ITEM_OK = 0, ITEM_LOST = 1;  // kernel-0 status; negative = OP
 struct PfState {  // post-filter parameters of the previous frame
     int32_t period, tapset;
     float gain;
-    int32_t pad;
+    int32_t lm1;  // 1 + LM of the stream's last decoded (not concealed) CELT frame, 0 = none yet
 };
 
 // Frame header, range decode -> frame kernel: one uint4 per stream.
@@ -116,6 +116,7 @@ struct MixArgs {  // k_mix_key / k_mix_place
     int channels, n_groups;          // n_groups = 1 or MIX_GROUPS
     uint32_t capacity;               // samples per channel the caller's rows hold (frame_size argument)
     uint8_t *last_lm;                // [n_streams] LM of the stream's last decoded packet, MIX_NO_ITEM = none yet (state)
+    const PfState *pf;               // [n_streams] or nullptr: after other CELT steps, last_lm is first taken from PfState::lm1
     uint8_t *key;                    // [n_streams] scratch: g*4 + lm, or MIX_NO_ITEM
     uint32_t *rank;                  // [n_streams] scratch: position inside the bucket
     MixPlan *plan;                   // zeroed before k_mix_key

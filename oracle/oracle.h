@@ -246,6 +246,22 @@ double orc_synth_bench(const uint8_t *packets, uint32_t n_streams, uint32_t n_fr
                        float *pcm_last /* [n_streams][frame*channels] or NULL */,
                        uint32_t *final_rng_xor);
 
+/* ---- one step of a batch (oracle/step.c): every stream advanced by one packet, n_threads threads over contiguous stream
+ * ranges.  states: [n_streams]; packets: row s at packets + s * pkt_stride, TOC first, lens[s] bytes (0 = lost); pcm_out: row s
+ * at pcm_out + s * pcm_stride floats, interleaved; final_rng: [n_streams], 0 for a lost frame.  The CELT steps take each
+ * stream's frame size (lm[s]: 120 << lm[s] samples, a lost frame conceals one frame of that size) and write hist[s] (or NULL),
+ * the comb history samples the GPU frame kernel counts for the frame: channels * (max(T_old, T_new, 15) + 2) when the
+ * post-filter runs, else 0.  The SILK step reads bandwidth and coded channel count from each TOC.  Returns 0 or the first
+ * error of a per-stream decode. */
+int orc_synth_step(orc_synth_state *states, uint32_t n_streams, const uint8_t *packets, size_t pkt_stride, const uint32_t *lens,
+                   const uint8_t *lm, int channels, int apply_comb, int n_threads, float *pcm_out, size_t pcm_stride,
+                   uint32_t *final_rng, uint32_t *hist);
+int orc_celt2_step(orc_synth_state *states, uint32_t n_streams, const uint8_t *packets, size_t pkt_stride, const uint32_t *lens,
+                   const uint8_t *lm, int channels, int apply_comb, int n_threads, float *pcm_out, size_t pcm_stride,
+                   uint32_t *final_rng, uint32_t *hist);
+int orc_silk_step(orc_silk_state *states, uint32_t n_streams, const uint8_t *packets, size_t pkt_stride, const uint32_t *lens,
+                  int frame_ms, int channels, int n_threads, float *pcm_out, size_t pcm_stride, uint32_t *final_rng);
+
 #ifdef __cplusplus
 }
 #endif

@@ -172,6 +172,9 @@ def lib():
     sig("orc_silk_packet", C.c_int, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_int, u32, u32, vp)
     sig("orc_silk_fill", C.c_int, C.c_uint64, u32, C.c_uint64, u32, C.c_int, C.c_int, C.c_int, u32, u32, C.c_int, vp)
     sig("orc_silk_bench", C.c_double, vp, u32, u32, u32, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.POINTER(u32))
+    for name in ("orc_synth_step", "orc_celt2_step"):
+        sig(name, C.c_int, vp, u32, vp, sz, vp, vp, C.c_int, C.c_int, C.c_int, vp, sz, vp, vp)
+    sig("orc_silk_step", C.c_int, vp, u32, vp, sz, vp, C.c_int, C.c_int, C.c_int, vp, sz, vp)
     _lib = L
     return L
 
@@ -327,6 +330,63 @@ class SynthStream:
         r = lib().orc_synth_decode_frame(C.byref(self.state), None, 0, lm, self.channels, int(self.apply_comb), C.byref(side), None, None, ptr(pcm))
         assert r == nf
         return pcm
+
+
+def _threads():
+    return min(len(os.sched_getaffinity(0)), 64)
+
+
+class CeltBatch:
+    """Oracle side of a batch of SYNTH-CELT/1 (bitstream 1) or /2 decoders, every stream advanced by one packet per step
+    (orc_synth_step / orc_celt2_step, multithreaded).  Stream s decodes exactly as a SynthStream / Celt2Stream would."""
+
+    def __init__(self, n_streams, channels, bitstream=1, apply_comb=True, n_threads=None):
+        self.n, self.channels, self.apply_comb = n_streams, channels, apply_comb
+        self.n_threads = n_threads or _threads()
+        self.fn = lib().orc_synth_step if bitstream == 1 else lib().orc_celt2_step
+        self.states = (SynthState * n_streams)()
+        for s in range(n_streams):
+            lib().orc_synth_state_init(C.byref(self.states[s]))
+
+    def step(self, packets, lens, lm, cap=None):
+        """packets uint8 [n, stride] (TOC first); lens [n] (0 = lost); lm: int or [n] -> (pcm float32 [n, cap * C] (cap: samples
+        per channel, default 120 << max lm), the frame at the start of each row, zeros after it; final_rng uint32 [n], 0 for a
+        lost frame; hist uint32 [n], the comb history samples the frame kernel counts for each frame)"""
+        packets = np.ascontiguousarray(packets, np.uint8)
+        lens = np.ascontiguousarray(lens, np.uint32)
+        lm = np.ascontiguousarray(np.broadcast_to(lm, (self.n,)), np.uint8)
+        assert packets.shape[0] == self.n and lens.shape == (self.n,)
+        pcm = np.zeros((self.n, (cap or 120 << int(lm.max())) * self.channels), np.float32)
+        rng = np.zeros(self.n, np.uint32)
+        hist = np.zeros(self.n, np.uint32)
+        rc = self.fn(self.states, self.n, ptr(packets), packets.shape[1], ptr(lens), ptr(lm), self.channels, int(self.apply_comb),
+                     self.n_threads, ptr(pcm), pcm.shape[1], ptr(rng), ptr(hist))
+        assert rc == 0, rc
+        return pcm, rng, hist
+
+
+class SilkBatch:
+    """Oracle side of a batch of SYNTH-SILK/1 decoders of `channels` channels, every stream advanced by one packet per step
+    (orc_silk_step, multithreaded; bandwidth and coded channel count from each packet's TOC)."""
+
+    def __init__(self, n_streams, channels, n_threads=None):
+        self.n, self.channels = n_streams, channels
+        self.n_threads = n_threads or _threads()
+        self.states = (SilkState * n_streams)()
+        for s in range(n_streams):
+            lib().orc_silk_state_init(C.byref(self.states[s]))
+
+    def step(self, packets, lens, frame_ms):
+        """-> (pcm float32 [n, frame_ms * 48 * C], final_rng uint32 [n], 0 for a lost frame)"""
+        packets = np.ascontiguousarray(packets, np.uint8)
+        lens = np.ascontiguousarray(lens, np.uint32)
+        assert packets.shape[0] == self.n and lens.shape == (self.n,)
+        pcm = np.zeros((self.n, frame_ms * 48 * self.channels), np.float32)
+        rng = np.zeros(self.n, np.uint32)
+        rc = lib().orc_silk_step(self.states, self.n, ptr(packets), packets.shape[1], ptr(lens), frame_ms, self.channels, self.n_threads,
+                                 ptr(pcm), pcm.shape[1], ptr(rng))
+        assert rc == 0, rc
+        return pcm, rng
 
 
 def silk_fill(first_stream, n_streams, first_frame, n_frames, bandwidth, frame_ms, channels, pkt_bytes, n_threads=1, lbrr_permille=0):
