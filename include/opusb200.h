@@ -138,7 +138,9 @@ typedef struct {
                                   * a stream's PCM row in samples per channel, as for Decoder::decode_float, and
                                   * result_per_stream[i] the samples stream i decoded (OPN_ERR_FRAME_SIZE_TOO_SMALL if its
                                   * frame does not fit).  A lost packet (lens[i] == 0) conceals one frame of the size of
-                                  * the stream's previous packet.  The step's buckets are built on the device. */
+                                  * the stream's previous packet, whichever kind of call decoded it; a PLC/DTX packet (the
+                                  * TOC alone or with one byte of payload) is concealed too, but sets that size from its
+                                  * TOC, as any packet does.  The step's buckets are built on the device. */
 
 #define OPN_FLAG_SILK_FRAMES 32u  /* with DEVICE_PTRS: every packet of the step is a single SILK-only frame of frame_size samples
                                   * (480 or 960 at 48 kHz) of the batch's channel count; the bandwidth (NB/MB/WB) is read from each
@@ -183,7 +185,9 @@ int opn_batch_wait(opn_batch *b, int ticket);
 /* Per-stream Decoder::final_range() of the last decoded frame (host buffer, n_streams words). */
 int opn_batch_final_ranges(opn_batch *b, uint32_t *out);
 /* Device-resident PCM ring (history + output): base pointer, samples per channel in the ring,
- * and the per-stream write position after the last call (device pointer, n_streams words). */
+ * and the per-stream write position after the last call (device pointer, n_streams words).  The ring holds the PCM
+ * before the decoder gain (opn_config.gain_q8): it is also the post-filter's history.  Only the dense PCM rows are
+ * scaled; a caller of OPN_FLAG_NO_PCM_COPY applies the gain itself. */
 int opn_batch_ring(opn_batch *b, float **ring, uint32_t *ring_samples, uint32_t **ring_pos_dev);
 /* Counters for the measurement harness.  kernel_ms[k]/kernel_launches[k]: k = 0 range decode (k_synth_rangedec),
  * 1 frame kernel (k_frame_w: PVQ expansion + IMDCT + TDAC + comb post-filter + PCM store; a large batch runs it as three

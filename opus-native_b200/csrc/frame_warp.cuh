@@ -419,7 +419,7 @@ __device__ __forceinline__ void frame_cta(const FrameArgs &A, uint32_t first_ite
         nw.period = t1;
         nw.tapset = tap1;
         nw.gain = g1;
-        nw.lm1 = lost ? old.lm1 : LM + 1;  // the frame size a mixed-frame step conceals a lost packet with (k_mix_key)
+        nw.lm1 = (lost && !(hdr.x & HDR_DTX)) ? old.lm1 : LM + 1;  // the size the stream conceals a loss with (k_mix_key, host path)
         A.pf[stream] = nw;
         if (A.result) A.result[stream] = NF;
         if (A.final_range) A.final_range[stream] = lost ? 0u : hdr.y;
@@ -455,7 +455,8 @@ template <int C, int MODE> __global__ void __launch_bounds__(32 * FRAME_WARPS, F
 // ---- bucketing of a mixed-frame step (MixPlan, opn_internal.h)
 // k_mix_key: one thread per stream reads its packet's TOC (the checks a host caller makes with query_packet_*,
 // src/lib.rs:219-325), picks the bucket and takes a position in it.  Streams of a warp that fall into the same bucket
-// take their positions with one atomic.  A lost packet (len 0) conceals one frame of the stream's previous size.
+// take their positions with one atomic.  A lost packet (len 0) conceals one frame of the stream's previous size; any packet,
+// PLC/DTX ones (TOC-only, one-byte payload) included, sets that size from its TOC.
 __global__ void __launch_bounds__(256) k_mix_key(MixArgs A)
 {
     const uint32_t s = blockIdx.x * 256u + threadIdx.x;
@@ -493,7 +494,7 @@ __global__ void __launch_bounds__(256) k_mix_key(MixArgs A)
                 if (g + 1u < G && (uint32_t)(((uint64_t)A.n_streams * (g + 1u)) / G) <= s) g += 1u;
             }
             key = g * 4u + (uint32_t)lm;
-            if (len > 1u) A.last_lm[s] = (uint8_t)lm;  // len <= 1 is PLC/DTX (decoder.rs:467): the size is not taken from it
+            if (len > 0u) A.last_lm[s] = (uint8_t)lm;
         }
     }
     const uint32_t peers = __match_any_sync(0xFFFFFFFFu, key);

@@ -205,6 +205,8 @@ struct opn_batch {
     unsigned long long *d_hist_samples = nullptr;  // measurement: history samples the post-filter needed (timed passes only)
     // host mirrors of DecoderInner fields (decoder.rs:236-258), per stream
     std::vector<int32_t> last_nf, bandwidth, last_duration, have_mode;
+    // device-resident steps ran since the last host-buffer call: have_mode / last_nf / silk_cs are behind the device state
+    bool dev_steps = false;
     // measurement
     bool timing = false;
     EventRing ev[3];
@@ -502,6 +504,7 @@ int run_silk_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offs
     a.result = d_result;
     a.final_range = b->d_final;
     a.softclip_reset = softclip_reset ? b->d_softclip : nullptr;
+    a.pf = b->d_pf;
     int rc = range_decode(b, p, [&](cudaStream_t st) { return launch_silk_rangedec(a, st); });
     if (rc) return rc;
     // Groups as for the CELT frame kernel: the serial LPC phase of one group's CTAs then overlaps the parallel phases of the
@@ -622,6 +625,32 @@ int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, c
         m.group = g;
         return launch_frame_mix(m, group_first(b->n, g + 1, G) - group_first(b->n, g, G), st);
     });
+}
+
+// Device-resident steps keep what the host path conceals with on the device: a stream's frame size in PfState::lm1, the
+// rate and coded channels of its last SILK frame in the SILK state.  Before the first host-buffer call after such steps,
+// the host mirrors are brought up to date from there.  Device-resident steps do not switch a stream between CELT and
+// SILK, so a stream that already has a mode keeps it; one that had none takes SILK when a SILK frame was decoded, CELT
+// when a CELT frame kernel recorded a size.
+int sync_host_state(opn_batch *b)
+{
+    if (!b->dev_steps) return OPN_OK;
+    const size_t n = b->n;
+    std::vector<PfState> pf(n);
+    std::vector<uint8_t> fs(b->silk ? 2 * n : 0);
+    const int rc = join_groups(b);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(pf.data(), b->d_pf, n * sizeof(PfState), cudaMemcpyDeviceToHost, b->stream));
+    if (b->silk) CU(cudaMemcpyAsync(fs.data(), b->d_silk.fs, 2 * n, cudaMemcpyDeviceToHost, b->stream));
+    CU(cudaStreamSynchronize(b->stream));
+    for (size_t i = 0; i < n; i++) {
+        const bool silk_frame = b->silk && fs[2 * i] != 0;
+        if (!b->have_mode[i] && (silk_frame || pf[i].lm1 > 0)) b->have_mode[i] = 1 + (silk_frame ? OPN_MODE_SILK : OPN_MODE_CELT);
+        if (silk_frame && b->have_mode[i] == 1 + OPN_MODE_SILK) b->silk_cs[i] = fs[2 * i + 1];
+        if (pf[i].lm1 > 0) b->last_nf[i] = 120 << (pf[i].lm1 - 1);
+    }
+    b->dev_steps = false;
+    return OPN_OK;
 }
 
 // PLC sizing of decode_native(None)/decode_frame(None), src/decoder.rs:427-441 and 467-513.
@@ -905,6 +934,7 @@ int opn_batch_reset(opn_batch *b)  // DecoderInner::reset, decoder.rs:286-303, f
     std::fill(b->last_duration.begin(), b->last_duration.end(), -1);
     std::fill(b->have_mode.begin(), b->have_mode.end(), 0);
     std::fill(b->silk_cs.begin(), b->silk_cs.end(), 0);
+    b->dev_steps = false;
     return OPN_OK;
 }
 
@@ -919,6 +949,8 @@ static int batch_decode_host(opn_batch *b, const uint8_t *arena, const uint32_t 
     Range nv_call("opn: host-buffer call (parse, upload, decode, download)");
     const uint32_t n = b->n;
     const int C = b->cfg.channels;
+    int rc = sync_host_state(b);
+    if (rc) return rc;
     // pre-pass: bytes to upload and an upper bound of the number of frames (items)
     size_t arena_end = 0, items_ub = 0;
     for (uint32_t i = 0; i < n; i++) {
@@ -940,7 +972,7 @@ static int batch_decode_host(opn_batch *b, const uint8_t *arena, const uint32_t 
     }
     const size_t esize = pcm_conv ? opn_sample_size(sample_format) : 0;
     if (pcm_conv && esize == 0) return OPN_ERR_BAD_ARG;
-    int rc = batch_alloc_staging(b, g, arena_end, items_ub, dense_stride, esize);
+    rc = batch_alloc_staging(b, g, arena_end, items_ub, dense_stride, esize);
     if (rc) return rc;
     const bool want_pcm = (pcm != nullptr || pcm_conv != nullptr) && !(flags & OPN_FLAG_NO_PCM_COPY);
     if (arena_end) CU(cudaMemcpyAsync(g.d_arena, arena, arena_end, cudaMemcpyHostToDevice, b->stream_up));
@@ -1224,6 +1256,7 @@ int opn_batch_decode_float(opn_batch *b, const uint8_t *arena, const uint32_t *o
     // decodes whatever single frame its packet holds.
     if (!arena) return OPN_ERR_BAD_ARG;
     if (b->cfg.bitstream == OPN_BITSTREAM_OPUS && !(flags & OPN_FLAG_SILK_FRAMES)) return OPN_ERR_UNIMPLEMENTED;  // celt/decoder.rs:47-56 is todo!()
+    b->dev_steps = true;
     float *dense = (flags & OPN_FLAG_NO_PCM_COPY) ? nullptr : pcm;
     if (dense && (pcm_stride_floats < std::min<size_t>(frame_size, 960) * (size_t)C || (pcm_stride_floats & 3) ||
                   (reinterpret_cast<uintptr_t>(dense) & 15)))

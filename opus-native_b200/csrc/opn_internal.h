@@ -31,12 +31,19 @@ constexpr int32_t ITEM_OK = 0, ITEM_LOST = 1;  // kernel-0 status; negative = OP
 struct PfState {  // post-filter parameters of the previous frame
     int32_t period, tapset;
     float gain;
-    int32_t lm1;  // 1 + LM of the stream's last decoded (not concealed) CELT frame, 0 = none yet
+    // 1 + LM of the frame size the stream conceals a loss with, 0 = no packet yet: the size of its last frame that came from
+    // a packet, decoded or PLC/DTX (a TOC with a payload of at most one byte: libopus takes st->frame_size from the TOC
+    // before it decodes the frames).  Written by every CELT frame kernel and by the SILK frame kernel (960 -> 4, 480 -> 3).
+    int32_t lm1;
 };
 
 // Frame header, range decode -> frame kernel: one uint4 per stream.
 //   .x = silence | postfilter << 1 | transient << 2 | intra << 3 | tapset << 4 | gain_idx << 8 | octave << 12 | period << 16
 //   .y = final range (Decoder::final_range), .z = tell_frac, .w = number of pulses
+// A lost item's header is zero but for HDR_DTX in .x: the item came from a packet (PLC/DTX), so it sets PfState::lm1.  On
+// the host path an item came from a packet when its offset is not 0: a concealed frame has offset 0, a parsed frame starts
+// after its packet's TOC.
+constexpr uint32_t HDR_DTX = 1u << 15;
 __host__ __device__ inline uint32_t hdr_pack(uint32_t silence, uint32_t postfilter, uint32_t transient, uint32_t intra, uint32_t tapset,
                                              uint32_t gain_idx, uint32_t octave, uint32_t period)
 {
@@ -115,7 +122,7 @@ struct MixArgs {  // k_mix_key / k_mix_place
     uint32_t n_streams;
     int channels, n_groups;          // n_groups = 1 or MIX_GROUPS
     uint32_t capacity;               // samples per channel the caller's rows hold (frame_size argument)
-    uint8_t *last_lm;                // [n_streams] LM of the stream's last decoded packet, MIX_NO_ITEM = none yet (state)
+    uint8_t *last_lm;                // [n_streams] LM of the stream's last packet (decoded or PLC/DTX), MIX_NO_ITEM = none yet (state)
     const PfState *pf;               // [n_streams] or nullptr: after other CELT steps, last_lm is first taken from PfState::lm1
     uint8_t *key;                    // [n_streams] scratch: g*4 + lm, or MIX_NO_ITEM
     uint32_t *rank;                  // [n_streams] scratch: position inside the bucket
@@ -177,6 +184,7 @@ struct SilkArgs {
     int32_t *result;
     uint32_t *final_range;
     float *softclip_reset;
+    PfState *pf;           // [n_streams] or nullptr: the frame kernel records the frame size in PfState::lm1
     // operator entry / tests (indexed by stream)
     opn_silk_side *side;   // or nullptr
     int32_t *exc_out;      // [n_streams][2][SILK_MAX_FRAME] or nullptr

@@ -58,6 +58,7 @@ __global__ void __launch_bounds__(32) k_silk_rangedec(SilkArgs A)
     const uint32_t stream = A.stream_idx ? A.stream_idx[item] : item;
     uint32_t len = A.lens[item];
     const uint8_t *src = A.arena + A.offsets[item];
+    const uint32_t dtx = (A.has_toc ? len > 0u : A.offsets[item] != 0u) ? HDR_DTX : 0u;  // a lost item of a packet: PLC/DTX
     int32_t status = len == 0u ? ITEM_LOST : ITEM_OK;
     int bandwidth = A.bandwidth;
     if (A.has_toc && len > 0u) {
@@ -75,7 +76,7 @@ __global__ void __launch_bounds__(32) k_silk_rangedec(SilkArgs A)
     if (status == ITEM_OK && len <= 1u) status = ITEM_LOST;  // decoder.rs:467
     A.status[stream] = status;
     if (status != ITEM_OK) {
-        if (status == ITEM_LOST) A.hdr[stream] = make_uint4(0u, 0u, 0u, 0u);
+        if (status == ITEM_LOST) A.hdr[stream] = make_uint4(dtx, 0u, 0u, 0u);
         return;
     }
     const int fs_khz = bandwidth == 0 ? 8 : bandwidth == 1 ? 12 : 16;
@@ -90,7 +91,7 @@ __global__ void __launch_bounds__(32) k_silk_rangedec(SilkArgs A)
     const uint32_t lbrr = d.bit_logp(1u);
     if (A.fec && !lbrr) {  // FEC asked of a packet that has none: conceal
         A.status[stream] = ITEM_LOST;
-        A.hdr[stream] = make_uint4(0u, 0u, 0u, 0u);
+        A.hdr[stream] = make_uint4(HDR_DTX, 0u, 0u, 0u);
         if (A.side) A.side[stream].lbrr = 0;
         return;
     }
@@ -540,6 +541,7 @@ template <int CS, int C> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k
                 A.st.fs[2 * stream] = (uint8_t)fs_khz;
                 A.st.fs[2 * stream + 1] = (uint8_t)CS;
             }
+            if (A.pf && (!lost || (A.hdr[stream].x & HDR_DTX))) A.pf[stream].lm1 = nb_subfr == 4 ? 4 : 3;
             if (A.result) A.result[stream] = n48;
             if (A.final_range) A.final_range[stream] = lost ? 0u : A.hdr[stream].y;
             if (A.softclip_reset && !lost) *reinterpret_cast<float2 *>(A.softclip_reset + 2 * (size_t)stream) = make_float2(0.f, 0.f);

@@ -310,6 +310,7 @@ __global__ void __launch_bounds__(RANGEDEC_WARPS_PER_CTA * 32) k_synth_rangedec(
     const uint32_t stream = A.stream_idx ? A.stream_idx[item] : item;
     uint32_t len = A.lens[item];
     const uint8_t *src = A.arena + A.offsets[item];
+    const bool from_packet = A.has_toc ? len > 0u : A.offsets[item] != 0u;  // a lost item of a packet is PLC/DTX (HDR_DTX)
 
     int32_t status = len == 0u ? ITEM_LOST : ITEM_OK;
     if (A.has_toc && len > 0u) {
@@ -334,7 +335,7 @@ __global__ void __launch_bounds__(RANGEDEC_WARPS_PER_CTA * 32) k_synth_rangedec(
     if (status == ITEM_LOST) {
         if (sd)
             for (uint32_t i = 0; i < SIDE_WORDS; i++) sw[i] = 0u;
-        A.hdr[stream] = make_uint4(0u, 0u, 0u, 0u);
+        A.hdr[stream] = make_uint4(from_packet ? HDR_DTX : 0u, 0u, 0u, 0u);
         return;
     }
     LaneDec d;
@@ -601,6 +602,7 @@ __global__ void __launch_bounds__(RANGEDEC_WARPS_PER_CTA * 32, OPN_C2_RD_MIN_CTA
     const uint32_t stream = A.stream_idx ? A.stream_idx[item] : item;
     uint32_t len = A.lens[item];
     const uint8_t *src = A.arena + A.offsets[item];
+    const bool from_packet = A.has_toc ? len > 0u : A.offsets[item] != 0u;
     int32_t status = len == 0u ? ITEM_LOST : ITEM_OK;
     if (A.has_toc && len > 0u) {
         const uint32_t toc = __ldg(src);
@@ -619,7 +621,7 @@ __global__ void __launch_bounds__(RANGEDEC_WARPS_PER_CTA * 32, OPN_C2_RD_MIN_CTA
     }
     if (status != ITEM_OK) {
         A.status[stream] = status;
-        if (status == ITEM_LOST) A.hdr[stream] = make_uint4(0u, 0u, 0u, 0u);
+        if (status == ITEM_LOST) A.hdr[stream] = make_uint4(from_packet ? HDR_DTX : 0u, 0u, 0u, 0u);
         return;
     }
     LaneCoder ec;

@@ -252,7 +252,9 @@ double orc_synth_bench(const uint8_t *packets, uint32_t n_streams, uint32_t n_fr
  * stream's frame size (lm[s]: 120 << lm[s] samples, a lost frame conceals one frame of that size) and write hist[s] (or NULL),
  * the comb history samples the GPU frame kernel counts for the frame: channels * (max(T_old, T_new, 15) + 2) when the
  * post-filter runs, else 0.  The SILK step reads bandwidth and coded channel count from each TOC.  Returns 0 or the first
- * error of a per-stream decode. */
+ * error of a per-stream decode.  lens[s] == ORC_STEP_SKIP leaves stream s out of the step: its state stays untouched and
+ * its row, final_rng and hist entries are not written. */
+#define ORC_STEP_SKIP 0xFFFFFFFFu
 int orc_synth_step(orc_synth_state *states, uint32_t n_streams, const uint8_t *packets, size_t pkt_stride, const uint32_t *lens,
                    const uint8_t *lm, int channels, int apply_comb, int n_threads, float *pcm_out, size_t pcm_stride,
                    uint32_t *final_rng, uint32_t *hist);

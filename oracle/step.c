@@ -7,7 +7,9 @@
  * otherwise (orc_synth_decode_frame, orc_celt2_decode_frame, orc_silk_decode_frame), so the results are the same bits.
  *
  * packets: row s at packets + s * pkt_stride, TOC first; lens[s] bytes of it, 0 = lost (so is a TOC-only packet,
- * src/decoder.rs:467).  pcm_out: row s at pcm_out + s * pcm_stride, the frame's interleaved samples; final_rng[s]: the range
+ * src/decoder.rs:467), ORC_STEP_SKIP = the stream takes no part in this step: its state stays untouched, its row and
+ * final_rng are not written (a host-buffer call that conceals several frames for some streams is modelled as several
+ * steps, each over the streams that still have a frame to go).  pcm_out: row s at pcm_out + s * pcm_stride, the frame's interleaved samples; final_rng[s]: the range
  * coder's final state, 0 for a lost frame. */
 #include "oracle.h"
 
@@ -36,6 +38,7 @@ static int max3(int a, int b, int c)
 
 static void celt_stream(step_job *j, uint32_t s)
 {
+    if (j->lens[s] == ORC_STEP_SKIP) return;
     orc_synth_state *st = (orc_synth_state *)j->states + s;
     const uint8_t *pkt = j->packets + (size_t)s * j->pkt_stride;
     const uint32_t len = j->lens[s] ? j->lens[s] - 1u : 0u; /* byte 0 is the TOC */
@@ -69,6 +72,7 @@ static void celt_stream(step_job *j, uint32_t s)
 
 static void silk_stream(step_job *j, uint32_t s)
 {
+    if (j->lens[s] == ORC_STEP_SKIP) return;
     orc_silk_state *st = (orc_silk_state *)j->states + s;
     const uint8_t *pkt = j->packets + (size_t)s * j->pkt_stride;
     const uint32_t len = j->lens[s] ? j->lens[s] - 1u : 0u;
@@ -129,7 +133,8 @@ static int celt_step(int kind, orc_synth_state *states, uint32_t n_streams, cons
 {
     if (!states || !packets || !lens || !lm || !pcm_out || !final_rng || channels < 1 || channels > 2) return ORC_ERR_BAD_ARG;
     for (uint32_t s = 0; s < n_streams; s++)
-        if (lm[s] > 3 || (size_t)(120 << lm[s]) * (size_t)channels > pcm_stride || lens[s] > pkt_stride) return ORC_ERR_BAD_ARG;
+        if (lm[s] > 3 || (size_t)(120 << lm[s]) * (size_t)channels > pcm_stride || (lens[s] > pkt_stride && lens[s] != ORC_STEP_SKIP))
+            return ORC_ERR_BAD_ARG;
     step_job j = {0};
     j.kind = kind;
     j.states = states;
@@ -168,7 +173,7 @@ int orc_silk_step(orc_silk_state *states, uint32_t n_streams, const uint8_t *pac
     if (!states || !packets || !lens || !pcm_out || !final_rng || channels < 1 || channels > 2) return ORC_ERR_BAD_ARG;
     if ((frame_ms != 10 && frame_ms != 20) || (size_t)frame_ms * 48u * (size_t)channels > pcm_stride) return ORC_ERR_BAD_ARG;
     for (uint32_t s = 0; s < n_streams; s++)
-        if (lens[s] > pkt_stride) return ORC_ERR_BAD_ARG;
+        if (lens[s] > pkt_stride && lens[s] != ORC_STEP_SKIP) return ORC_ERR_BAD_ARG;
     step_job j = {0};
     j.kind = 2;
     j.states = states;

@@ -332,6 +332,16 @@ class SynthStream:
         return pcm
 
 
+STEP_SKIP = 0xFFFFFFFF  # ORC_STEP_SKIP
+
+
+def _with_skip(lens, skip):
+    lens = np.array(lens, np.uint32)
+    if skip is not None:
+        lens[np.asarray(skip, bool)] = STEP_SKIP
+    return lens
+
+
 def _threads():
     return min(len(os.sched_getaffinity(0)), 64)
 
@@ -348,12 +358,13 @@ class CeltBatch:
         for s in range(n_streams):
             lib().orc_synth_state_init(C.byref(self.states[s]))
 
-    def step(self, packets, lens, lm, cap=None):
-        """packets uint8 [n, stride] (TOC first); lens [n] (0 = lost); lm: int or [n] -> (pcm float32 [n, cap * C] (cap: samples
-        per channel, default 120 << max lm), the frame at the start of each row, zeros after it; final_rng uint32 [n], 0 for a
-        lost frame; hist uint32 [n], the comb history samples the frame kernel counts for each frame)"""
+    def step(self, packets, lens, lm, cap=None, skip=None):
+        """packets uint8 [n, stride] (TOC first); lens [n] (0 = lost); lm: int or [n]; skip: bool [n] or None, streams left out
+        of the step (state untouched, row, final_rng and hist zero) -> (pcm float32 [n, cap * C] (cap: samples per channel,
+        default 120 << max lm), the frame at the start of each row, zeros after it; final_rng uint32 [n], 0 for a lost frame;
+        hist uint32 [n], the comb history samples the frame kernel counts for each frame)"""
         packets = np.ascontiguousarray(packets, np.uint8)
-        lens = np.ascontiguousarray(lens, np.uint32)
+        lens = _with_skip(lens, skip)
         lm = np.ascontiguousarray(np.broadcast_to(lm, (self.n,)), np.uint8)
         assert packets.shape[0] == self.n and lens.shape == (self.n,)
         pcm = np.zeros((self.n, (cap or 120 << int(lm.max())) * self.channels), np.float32)
@@ -376,10 +387,10 @@ class SilkBatch:
         for s in range(n_streams):
             lib().orc_silk_state_init(C.byref(self.states[s]))
 
-    def step(self, packets, lens, frame_ms):
-        """-> (pcm float32 [n, frame_ms * 48 * C], final_rng uint32 [n], 0 for a lost frame)"""
+    def step(self, packets, lens, frame_ms, skip=None):
+        """skip as for CeltBatch.step -> (pcm float32 [n, frame_ms * 48 * C], final_rng uint32 [n], 0 for a lost frame)"""
         packets = np.ascontiguousarray(packets, np.uint8)
-        lens = np.ascontiguousarray(lens, np.uint32)
+        lens = _with_skip(lens, skip)
         assert packets.shape[0] == self.n and lens.shape == (self.n,)
         pcm = np.zeros((self.n, frame_ms * 48 * self.channels), np.float32)
         rng = np.zeros(self.n, np.uint32)

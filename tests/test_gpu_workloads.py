@@ -243,14 +243,15 @@ def _mixed_packets(n, nsteps, rnd, channels, first=0):
 
 class MixedOracle:
     """Frame sizes of a mixed-frame step as a decoder sees them: a lost packet conceals one frame of the stream's previous
-    size, whatever kind of step decoded that (decoder.rs:427-441); before any packet, one frame of the row's capacity."""
+    size, whatever kind of step decoded that (decoder.rs:427-441); any packet of lens >= 1, PLC/DTX ones included, sets
+    that size from its TOC; before any packet, one frame of the row's capacity."""
 
     def __init__(self, n, cap_lm=3):
         self.last = np.full(n, cap_lm, np.uint8)
 
     def sizes(self, lens, lm):
         out = np.where(lens > 0, lm, self.last).astype(np.uint8)
-        self.last = np.where(lens > 1, lm, self.last).astype(np.uint8)
+        self.last = np.where(lens > 0, lm, self.last).astype(np.uint8)
         return out
 
 

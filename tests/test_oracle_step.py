@@ -103,3 +103,50 @@ def test_silk_step_equals_per_stream_decoders(channels):
             assert np.array_equal(pcm[s].view(np.uint32), want.view(np.uint32)), (f, s)
             assert rng[s] == (side.final_rng if lens[s] else 0), (f, s)
     assert np.abs(pcm).max() > 0.01
+
+
+@pytest.mark.parametrize("bitstream", [1, 2, 0])
+def test_skipped_streams_are_left_untouched(bitstream):
+    """skip: a stream left out of a step keeps its state, as a per-stream decoder that was not called (SYNTH-CELT/1, /2 and,
+    for bitstream 0, SYNTH-SILK/1); its row, final range and history count are zero.  A host-buffer call that conceals
+    several frames for some streams is modelled with such steps."""
+    rnd = np.random.default_rng(90 + bitstream)
+    channels = 2
+    if bitstream:
+        packets, lens, lm = _celt_packets(bitstream, rnd, channels)
+        batch = O.CeltBatch(NS, channels, bitstream, n_threads=4)
+        ref = [(O.SynthStream if bitstream == 1 else O.Celt2Stream)(3, channels) for _ in range(NS)]
+    else:
+        bws = rnd.integers(0, 3, NS)
+        packets = np.stack([O.silk_fill(200 + s, 1, 0, NSTEPS, int(bws[s]), 20, channels, 192)[:, 0] for s in range(NS)], axis=1)
+        lens = np.full((NSTEPS, NS), 192, np.uint32)
+        lens[1:][rnd.random((NSTEPS - 1, NS)) < 0.1] = 0
+        batch = O.SilkBatch(NS, channels, n_threads=4)
+        ref = [O.SilkStream(channels) for _ in range(NS)]
+    n_skipped = 0
+    for f in range(NSTEPS):
+        skip = rnd.random(NS) < 0.3
+        if bitstream:
+            pcm, rng, hist = batch.step(packets[f], lens[f], lm[f], cap=960, skip=skip)
+        else:
+            pcm, rng = batch.step(packets[f], lens[f], 20, skip=skip)
+            hist = np.zeros(NS, np.uint32)
+        for s in range(NS):
+            if skip[s]:
+                assert not pcm[s].any() and rng[s] == 0 and hist[s] == 0, (f, s)
+                n_skipped += 1
+                continue
+            payload = packets[f, s, 1:lens[f, s]] if lens[f, s] else b""
+            if bitstream == 1:
+                ref[s].lm = int(lm[f, s])
+                side, _, _, want = ref[s].decode(payload)
+            elif bitstream == 2:
+                ref[s].lm = int(lm[f, s])
+                side, want = ref[s].decode(payload)
+            else:
+                side, _, _, want = ref[s].decode(payload, int(bws[s]), 20, channels, lost=not lens[f, s])
+            assert np.array_equal(pcm[s, :len(want)].view(np.uint32), want.view(np.uint32)), (f, s)
+            assert rng[s] == (side.final_rng if lens[f, s] > 1 else 0), (f, s)
+    for s in range(NS):
+        assert bytes(batch.states[s]) == bytes(ref[s].state), s
+    assert n_skipped > NS
