@@ -140,7 +140,19 @@ typedef struct {
                                   * frame does not fit).  A lost packet (lens[i] == 0) conceals one frame of the size of
                                   * the stream's previous packet, whichever kind of call decoded it; a PLC/DTX packet (the
                                   * TOC alone or with one byte of payload) is concealed too, but sets that size from its
-                                  * TOC, as any packet does.  The step's buckets are built on the device. */
+                                  * TOC, as any packet does.  The step's buckets are built on the device.  SILK packets are
+                                  * OPN_ERR_UNIMPLEMENTED in this step; OPN_FLAG_MIXED_MODES takes them. */
+#define OPN_FLAG_MIXED_MODES 128u /* with DEVICE_PTRS, on a batch created with OPN_BITSTREAM_SYNTH_SILK_1 (else OPN_ERR_BAD_ARG; not with
+                                  * OPN_FLAG_SILK_FRAMES): OPN_FLAG_MIXED_FRAMES for CELT and SILK packets in one step.  Each stream
+                                  * takes a single-frame CELT packet (2.5-20 ms), a single-frame SILK-only packet (NB/MB/WB, 10 or
+                                  * 20 ms) or a loss; frame_size is the capacity of a row and result_per_stream[i] the samples stream
+                                  * i decoded, as for OPN_FLAG_MIXED_FRAMES.  A stream switches codec as Decoder::decode does: SILK
+                                  * after CELT resets the SILK decoder, the CELT decoder conceals 5 ms, which replace the first
+                                  * 2.5 ms of the row and cross-fade into the next 2.5 ms (decoder.rs:519-557, 765-788); CELT after
+                                  * SILK resets the CELT decoder (decoder.rs:703-705).  A loss conceals one frame of the stream's
+                                  * last size with the codec of its last packet.  Per-stream errors, state untouched:
+                                  * OPN_ERR_UNIMPLEMENTED for hybrid, 40/60 ms SILK, multi-frame packets, a foreign channel count and
+                                  * CELT packets of OPN_BITSTREAM_OPUS; OPN_ERR_FRAME_SIZE_TOO_SMALL when the frame does not fit. */
 
 #define OPN_FLAG_SILK_FRAMES 32u  /* with DEVICE_PTRS: every packet of the step is a single SILK-only frame of frame_size samples
                                   * (480 or 960 at 48 kHz) of the batch's channel count; the bandwidth (NB/MB/WB) is read from each
@@ -161,7 +173,8 @@ int opn_batch_reset(opn_batch *b);
  * Host-buffer calls take any mix of frame sizes, multi-frame packets and packets whose channel count differs from the
  * batch's (stream_channels, decoder.rs:332: a mono packet fills both channels of a stereo decoder, a stereo packet is
  * averaged into a mono decoder).  Device-resident calls (OPN_FLAG_DEVICE_PTRS) take single-frame packets of the batch's
- * channel count: all of frame_size samples, or of any size with OPN_FLAG_MIXED_FRAMES. */
+ * channel count: all of frame_size samples, or of any size with OPN_FLAG_MIXED_FRAMES; CELT and SILK packets in one call,
+ * with mode switches, take OPN_FLAG_MIXED_MODES. */
 int opn_batch_decode_float(opn_batch *b, const uint8_t *arena, const uint32_t *offsets,
                            const uint32_t *lens, float *pcm, size_t pcm_stride_floats,
                            size_t frame_size, int32_t *result_per_stream, uint32_t flags);
@@ -193,7 +206,8 @@ int opn_batch_ring(opn_batch *b, float **ring, uint32_t *ring_samples, uint32_t 
  * 1 frame kernel (k_frame_w: PVQ expansion + IMDCT + TDAC + comb post-filter + PCM store; a large batch runs it as three
  * concurrent launches over thirds of the streams, and kernel_ms[1] is the time from the first launch to the last
  * completion), 2 the two bucketing kernels of a mixed-frame step (k_mix_key, k_mix_place: counted, not timed; kernel_ms[2]
- * stays 0).  Timing must be enabled first (the stages of a step then run one after the other, with cudaEvents around
+ * stays 0).  A mixed-mode step counts its CELT and SILK range decodes under 0, its CELT and SILK frame kernels under 1,
+ * and its mode-switch launches (resets, fade) under 2; they run inside the frame stage's timed span.  Timing must be enabled first (the stages of a step then run one after the other, with cudaEvents around
  * each). */
 int opn_batch_enable_timing(opn_batch *b, int on);
 int opn_batch_stats(opn_batch *b, uint64_t kernel_launches[3], double kernel_ms[3], int reset);

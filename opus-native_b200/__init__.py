@@ -13,7 +13,7 @@ from ._capi import (  # noqa: F401
     DecoderConfiguration, Decoder, BatchDecoder, HostBuffer, host_register, host_unregister,
     op_rangedec_script, op_imdct_tdac, op_comb_filter_inplace, op_comb_filter, op_pcm_soft_clip, op_bitexact_trig, op_smooth_fade,
     op_synth_symbols, synth_packet, synth_fill, enc_run_script, op_celt2_symbols, celt2_packet, celt2_fill, CELT2_SIDE_DTYPE,
-    silk_fill, op_silk_frames, SILK_SIDE_DTYPE, SILK_MAX_FRAME, BITSTREAM_SYNTH_SILK_1, FLAG_SILK_FRAMES, FLAG_DECODE_FEC,
+    silk_fill, op_silk_frames, SILK_SIDE_DTYPE, SILK_MAX_FRAME, BITSTREAM_SYNTH_SILK_1, FLAG_SILK_FRAMES, FLAG_DECODE_FEC, FLAG_MIXED_MODES,
     OP_DTYPE, OUT_DTYPE, SIDE_DTYPE,
     OP_UINT, OP_BITS, OP_BIT_LOGP, OP_ICDF, OP_LAPLACE, OP_BIT_VIA_DECODE, OP_BIT_VIA_DECODE_BIN,
     OP_PULSES, OP_SHRINK, OP_TELL, OP_PULSES_EVENTS, FLAG_DEVICE_PTRS, FLAG_NO_PCM_COPY, FLAG_INPUTS_READY, FLAG_SUBMIT_ONLY, FLAG_MIXED_FRAMES,

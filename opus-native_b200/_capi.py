@@ -11,6 +11,7 @@ _SO = os.path.join(_HERE, "libopusb200.so")
 
 OP_UINT, OP_BITS, OP_BIT_LOGP, OP_ICDF, OP_LAPLACE, OP_BIT_VIA_DECODE, OP_BIT_VIA_DECODE_BIN, OP_PULSES, OP_SHRINK, OP_TELL, OP_PULSES_EVENTS = range(11)
 FLAG_DEVICE_PTRS, FLAG_NO_PCM_COPY, FLAG_INPUTS_READY, FLAG_SUBMIT_ONLY, FLAG_MIXED_FRAMES, FLAG_SILK_FRAMES, FLAG_DECODE_FEC = 1, 2, 4, 8, 16, 32, 64
+FLAG_MIXED_MODES = 128
 # OPN_BITSTREAM_*: CELT frames are Unimplemented (as in the crate, whose CeltDecoder::decode is todo!()) unless the caller
 # opts in to the synthetic SYNTH-CELT/1 frame layout (DESIGN.md section 3; not Opus-interoperable)
 BITSTREAM_OPUS, BITSTREAM_SYNTH_CELT_1, BITSTREAM_SYNTH_CELT_2 = 0, 1, 2

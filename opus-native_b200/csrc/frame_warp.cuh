@@ -457,30 +457,56 @@ template <int C, int MODE> __global__ void __launch_bounds__(32 * FRAME_WARPS, F
 // src/lib.rs:219-325), picks the bucket and takes a position in it.  Streams of a warp that fall into the same bucket
 // take their positions with one atomic.  A lost packet (len 0) conceals one frame of the stream's previous size; any packet,
 // PLC/DTX ones (TOC-only, one-byte payload) included, sets that size from its TOC.
+// A mixed-mode step (A.modes != 0) buckets SILK-only packets as well, by (group, 10 / 20 ms); a loss conceals with the codec
+// of the stream's last packet (PF_SILK in last_lm).  A packet of the other codec than the stream's last one is a mode switch,
+// listed for its group: CELT -> SILK also takes a 2.5 ms CELT concealment item (bucket (g, 1)), the start of the transition.
+__device__ __forceinline__ uint32_t mix_take(uint32_t key, uint32_t *counter)
+{
+    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, key);
+    uint32_t rank = 0u;
+    if (key != MIX_NO_ITEM) {
+        const int leader = __ffs(peers) - 1;
+        uint32_t base = 0u;
+        if ((int)(threadIdx.x & 31u) == leader) base = atomicAdd(counter, (uint32_t)__popc(peers));
+        base = __shfl_sync(peers, base, leader);
+        rank = base + (uint32_t)__popc(peers & ((1u << (threadIdx.x & 31u)) - 1u));
+    }
+    return rank;
+}
+
 __global__ void __launch_bounds__(256) k_mix_key(MixArgs A)
 {
     const uint32_t s = blockIdx.x * 256u + threadIdx.x;
     const bool on = s < A.n_streams;
-    uint32_t key = MIX_NO_ITEM;
+    uint32_t key = MIX_NO_ITEM, tkey = MIX_NO_ITEM;
     int32_t err = 0;
     if (on) {
-        if (A.pf) {  // after other CELT steps (their frame kernels have finished): they recorded each stream's last frame size
+        if (A.pf) {  // after other steps (their frame kernels have finished): they recorded each stream's last frame size and codec
             const int32_t l1 = A.pf[s].lm1;
-            A.last_lm[s] = l1 > 0 ? (uint8_t)(l1 - 1) : (uint8_t)MIX_NO_ITEM;
+            A.last_lm[s] = (l1 & PF_LM1) > 0 ? (uint8_t)(((l1 & PF_LM1) - 1) | (l1 & PF_SILK)) : (uint8_t)MIX_NO_ITEM;
         }
         const uint32_t len = A.lens[s];
+        const uint32_t l = A.last_lm[s];
         int lm = -1;
+        bool silk = false;
         if (len == 0u) {
-            const uint32_t l = A.last_lm[s];
             // nothing decoded yet: zeros for the caller's frame size (decoder.rs:473-484); the frame kernel produces
             // them from an empty spectrum and an empty overlap
-            lm = l != MIX_NO_ITEM ? (int)l : (A.capacity >= 960u ? 3 : A.capacity >= 480u ? 2 : A.capacity >= 240u ? 1 : 0);
+            lm = l != MIX_NO_ITEM ? (int)(l & 3u) : (A.capacity >= 960u ? 3 : A.capacity >= 480u ? 2 : A.capacity >= 240u ? 1 : 0);
+            silk = A.modes && l != MIX_NO_ITEM && (l & (uint32_t)PF_SILK);
         } else {
             const uint32_t toc = A.arena[A.offsets[s]];
-            if ((toc & 0x80u) == 0u) err = OPN_ERR_UNIMPLEMENTED;                  // SILK / hybrid
-            else if ((toc & 0x3u) != 0u) err = OPN_ERR_UNIMPLEMENTED;              // multi-frame packets: host path only
+            if ((toc & 0x3u) != 0u) err = OPN_ERR_UNIMPLEMENTED;                          // multi-frame packets: host path only
             else if (((toc & 0x4u) ? 2 : 1) != A.channels) err = OPN_ERR_UNIMPLEMENTED;  // mono<->stereo mapping
-            else lm = (int)((toc >> 3) & 0x3u);
+            else if (toc & 0x80u) {
+                if (A.modes == 2) err = OPN_ERR_UNIMPLEMENTED;                           // CELT frames of OPN_BITSTREAM_OPUS
+                else lm = (int)((toc >> 3) & 0x3u);
+            } else if (A.modes == 0 || (toc >> 3) >= 12u || ((toc >> 3) & 3u) > 1u) {
+                err = OPN_ERR_UNIMPLEMENTED;                                             // hybrid, 40 / 60 ms SILK
+            } else {
+                lm = ((toc >> 3) & 1u) ? 3 : 2;                                          // SILK 20 ms = 960, 10 ms = 480 samples
+                silk = true;
+            }
         }
         if (lm >= 0 && (120u << lm) > A.capacity) {
             err = OPN_ERR_FRAME_SIZE_TOO_SMALL;  // decoder.rs:388-390
@@ -488,23 +514,34 @@ __global__ void __launch_bounds__(256) k_mix_key(MixArgs A)
         }
         if (lm >= 0) {
             uint32_t g = 0u;  // group g holds the streams [floor(n g / G), floor(n (g+1) / G)), as a uniform bucket's launches do
-            if (A.n_groups > 1) {
-                const uint32_t G = (uint32_t)A.n_groups;
+            const uint32_t G = (uint32_t)A.n_groups;
+            if (G > 1u) {
                 g = (uint32_t)(((uint64_t)s * G) / A.n_streams);
                 if (g + 1u < G && (uint32_t)(((uint64_t)A.n_streams * (g + 1u)) / G) <= s) g += 1u;
             }
-            key = g * 4u + (uint32_t)lm;
-            if (len > 0u) A.last_lm[s] = (uint8_t)lm;
+            key = silk ? (uint32_t)MIX_KEY_SILK | (g * 2u + (uint32_t)(lm - 2)) : g * 4u + (uint32_t)lm;
+            if (len > 0u) {
+                // a mode switch (decoder.rs:519-557, 703-705): listed for the group's frame stream, never applied here
+                const bool was_silk = l != MIX_NO_ITEM && (l & (uint32_t)PF_SILK);
+                if (A.modes && l != MIX_NO_ITEM && silk != was_silk) {
+                    const uint32_t d = silk ? 0u : 1u;
+                    const uint32_t k = atomicAdd(&A.plan->nsw[g][d], 1u);
+                    A.sw[d * A.n_streams + (uint32_t)(((uint64_t)A.n_streams * g) / G) + k] = s;
+                    if (silk) tkey = g * 4u + 1u;
+                }
+                A.last_lm[s] = (uint8_t)(lm | (silk ? PF_SILK : 0));
+            }
         }
     }
-    const uint32_t peers = __match_any_sync(0xFFFFFFFFu, key);
-    uint32_t rank = 0u;
-    if (key != MIX_NO_ITEM) {
-        const int leader = __ffs(peers) - 1;
-        uint32_t base = 0u;
-        if ((int)(threadIdx.x & 31u) == leader) base = atomicAdd(&A.plan->count[key >> 2][key & 3u], (uint32_t)__popc(peers));
-        base = __shfl_sync(peers, base, leader);
-        rank = base + (uint32_t)__popc(peers & ((1u << (threadIdx.x & 31u)) - 1u));
+    uint32_t *counter = nullptr;
+    if (key != MIX_NO_ITEM) counter = (key & MIX_KEY_SILK) ? &A.plan->scount[(key & 31u) >> 1][key & 1u] : &A.plan->count[key >> 2][key & 3u];
+    const uint32_t rank = mix_take(key, counter);
+    if (A.modes) {
+        const uint32_t trank = mix_take(tkey, tkey != MIX_NO_ITEM ? &A.plan->count[tkey >> 2][1] : nullptr);
+        if (on && tkey != MIX_NO_ITEM) {
+            key |= MIX_KEY_TRANS;
+            A.rank[A.n_streams + s] = trank;
+        }
     }
     if (on) {
         A.key[s] = (uint8_t)key;
@@ -515,7 +552,7 @@ __global__ void __launch_bounds__(256) k_mix_key(MixArgs A)
 // k_mix_place: bucket starts from the counts (every CTA recomputes the dozen sums), then each stream's item record.
 __global__ void __launch_bounds__(256) k_mix_place(MixArgs A)
 {
-    __shared__ uint32_t s_start[MIX_GROUPS * 4];
+    __shared__ uint32_t s_start[MIX_GROUPS * 4], s_sstart[MIX_GROUPS * 2];
     if (threadIdx.x == 0) {
         uint32_t at = 0u;
         MixPlan &P = *A.plan;
@@ -535,17 +572,99 @@ __global__ void __launch_bounds__(256) k_mix_place(MixArgs A)
             if (blockIdx.x == 0) P.cta0[g][4] = cta;
         }
         if (blockIdx.x == 0) P.items_padded = at;
+        if (A.modes) {
+            const uint32_t per_cta = (uint32_t)(SILK_ROWS / A.channels);  // SILK packets have the batch's channel count
+            at = 0u;
+            for (int g = 0; g < MIX_GROUPS; g++) {
+                uint32_t cta = 0u;
+                for (int j = 0; j < 2; j++) {  // 20 ms first
+                    const int k = 1 - j;
+                    const uint32_t n = P.scount[g][k];
+                    s_sstart[g * 2 + k] = at;
+                    if (blockIdx.x == 0) {
+                        P.sstart[g][k] = at;
+                        P.scta0[g][j] = cta;
+                    }
+                    at += (n + SILK_PAD - 1u) / SILK_PAD * SILK_PAD;
+                    cta += (n + per_cta - 1u) / per_cta;
+                }
+                if (blockIdx.x == 0) P.scta0[g][2] = cta;
+            }
+        }
     }
     __syncthreads();
     const uint32_t s = blockIdx.x * 256u + threadIdx.x;
     if (s >= A.n_streams) return;
     const uint32_t key = A.key[s];
     if (key == MIX_NO_ITEM) return;
+    if (key & MIX_KEY_SILK) {
+        const uint32_t b = (key & 31u), item = s_sstart[b] + A.rank[s];
+        A.sitem_offsets[item] = A.offsets[s];
+        A.sitem_lens[item] = A.lens[s];
+        A.sitem_stream[item] = s;
+        A.sitem_ms[item] = (b & 1u) ? 20 : 10;
+        if (key & MIX_KEY_TRANS) {  // the CELT decoder's 2.5 ms concealment (a lost item) ahead of the stream's first SILK frame
+            const uint32_t t = s_start[(b >> 1) * 4 + 1] + A.rank[A.n_streams + s];
+            A.item_offsets[t] = 0u;
+            A.item_lens[t] = 0u;
+            A.item_stream[t] = s;
+            A.item_lm[t] = 1;
+        }
+        return;
+    }
     const uint32_t item = s_start[key] + A.rank[s];
     A.item_offsets[item] = A.offsets[s];
     A.item_lens[item] = A.lens[s];
     A.item_stream[item] = s;
     A.item_lm[item] = (uint8_t)(key & 3u);
+}
+
+// The mode switches of one group of a mixed-mode step (SwitchArgs), one warp per listed stream, on the group's frame stream.
+// Phase 0, before the group's frame kernels: CELT -> SILK streams start the SILK decoder from rest (silk_dec.reset(),
+// decoder.rs:555-557); SILK -> CELT streams reset the CELT decoder (decoder.rs:703-705): overlap carry, post-filter state and
+// the ring, the post-filter's history.
+// Phase 1, after them (dense rows only): the transition of decoder.rs:765-788.  The CELT concealment item wrote 2.5 ms into the
+// ring just ahead of the SILK frame, so both inputs are read back from the ring, where they sit before the decoder gain:
+// the first 2.5 ms of the row are the concealment, the next 2.5 ms smooth_fade_into_in2(concealment, SILK), then the gain.
+__global__ void __launch_bounds__(256) k_mode_switch(SwitchArgs A)
+{
+    const uint32_t lane = threadIdx.x & 31u;
+    const int C = A.channels;
+    const uint32_t n0 = A.plan->nsw[A.group][0], n1 = A.plan->nsw[A.group][1];
+    const uint32_t n = A.phase == 0 ? n0 + n1 : n0;
+    for (uint32_t w = blockIdx.x * 8u + (threadIdx.x >> 5); w < n; w += gridDim.x * 8u) {
+        const bool to_silk = w < n0;
+        const uint32_t s = A.sw[(to_silk ? 0u : A.n_streams) + A.first + (to_silk ? w : w - n0)];
+        if (A.phase == 0) {
+            if (to_silk) {
+                if (lane < 2u) A.silk_fs[2 * (size_t)s + lane] = 0;
+            } else {
+                float4 *ring = reinterpret_cast<float4 *>(A.ring + (size_t)s * RING_SAMPLES * C);
+                for (int i = (int)lane; i < RING_SAMPLES * C / 4; i += 32) ring[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+                float4 *carry = reinterpret_cast<float4 *>(A.carry + (size_t)s * C * 60);
+                if ((int)lane < 15 * C) carry[lane] = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (lane == 0) A.pf[s] = PfState{0, 0, 0.0f, 0};
+            }
+            continue;
+        }
+        // a SILK frame that was concealed before any SILK frame (a PLC/DTX packet) is silence and left the ring alone
+        const bool silent = A.silk_fs[2 * (size_t)s] == 0;
+        const int n48 = silent ? 0 : ((A.pf[s].lm1 & PF_LM1) == 4 ? 960 : 480);
+        const float *ring = A.ring + (size_t)s * RING_SAMPLES * C;
+        const int p0 = ((int)A.ring_pos[s] + 2 * RING_SAMPLES - n48 - 240) % RING_SAMPLES;  // the concealment's first sample
+        float *row = A.dense + (size_t)s * A.dense_stride;
+        const int f = 120 * C;
+        for (int j = (int)lane; j < f; j += 32) {
+            const int t = j / C, c = j - t * C;
+            const float tr0 = ring[(size_t)((p0 + t) % RING_SAMPLES) * C + c];
+            const float tr1 = ring[(size_t)((p0 + 120 + t) % RING_SAMPLES) * C + c];
+            const float sk = silent ? 0.0f : ring[(size_t)((p0 + 360 + t) % RING_SAMPLES) * C + c];
+            const float wv = g_tab.window[t];
+            const float wq = wv * wv;
+            row[j] = tr0 * A.gain;
+            row[f + j] = ((wq * sk) + ((1.0f - wq) * tr1)) * A.gain;
+        }
+    }
 }
 
 // Operator-level Mdct::backward on independent rows (tests; opn_op_imdct_tdac): one warp per row.

@@ -192,11 +192,23 @@ struct opn_batch {
     // other CELT steps first waits for their frame kernels and then takes d_last_lm from PfState::lm1.
     bool lm_pending = false;  // CELT steps other than mixed-frame ones ran since the last mixed-frame step's bucketing
     int lm_set = 0;
-    uint32_t *d_mix_rank = nullptr;                      // [n] scratch
+    // Mixed-mode steps (OPN_FLAG_MIXED_MODES) take each stream's codec from the same record (PF_SILK), so they also wait for
+    // SILK steps, uniform or host-path ones; they wait for the frame kernels of the last step of any kind (fr_set).
+    bool mode_pending = false;  // steps other than mixed-frame and mixed-mode ones ran since the last mixed-mode step's bucketing
+    int fr_set = 0;             // buffer set of the last step's frame kernels
+    uint32_t *d_mix_rank = nullptr;                      // [2n] scratch
     uint32_t *d_mix_items[NSETS] = {};                   // [3][mix_item_cap(n)]: offsets | lens | stream ids, by item
     uint8_t *d_mix_lm[NSETS] = {};                       // [mix_item_cap(n)]
     MixPlan *d_mix_plan[NSETS] = {};
     cudaEvent_t ev_mix[NSETS] = {};                      // buckets of set p are built
+    // mixed-mode steps, allocated on first use: the SILK item table and the mode switches of the step, and the SILK range
+    // decode's own frame headers and status.  A CELT -> SILK stream has a CELT concealment item and a SILK item in one step:
+    // with one hdr / status per stream, the SILK range decode would overwrite what the concealment reads.
+    uint32_t *d_mix_sitems[NSETS] = {};                  // [3][mix_silk_cap(n)]: offsets | lens | stream ids
+    uint8_t *d_mix_sms[NSETS] = {};                      // [mix_silk_cap(n)] frame duration, MIX_NO_ITEM = padding
+    uint32_t *d_mix_sw[NSETS] = {};                      // [2][n] streams that switch mode
+    uint4 *d_shdr[NSETS] = {};
+    int32_t *d_sstatus[NSETS] = {};
     // SYNTH-SILK/1 (OPN_BITSTREAM_SYNTH_SILK_1): per-stream filter state and one record set per range decode in flight
     bool silk = false;
     SilkState d_silk{};
@@ -207,6 +219,7 @@ struct opn_batch {
     std::vector<int32_t> last_nf, bandwidth, last_duration, have_mode;
     // device-resident steps ran since the last host-buffer call: have_mode / last_nf / silk_cs are behind the device state
     bool dev_steps = false;
+    bool silk_dev = false;  // mixed-mode steps among them: streams may have switched codec
     // measurement
     bool timing = false;
     EventRing ev[3];
@@ -400,6 +413,7 @@ template <class F> int frame_launches(opn_batch *b, int p, int G, F &&launch)
     CU(cudaEventRecord(b->ev_k1[p], b->stream));
     b->k1_recorded[p] = true;
     b->k1_grouped[p] = G > 1;
+    b->fr_set = p;
     return OPN_OK;
 }
 
@@ -465,6 +479,7 @@ int run_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, 
     if (rc) return rc;
     b->lm_pending = true;
     b->lm_set = p;
+    b->mode_pending = true;
     return OPN_OK;
 }
 
@@ -510,19 +525,32 @@ int run_silk_bucket(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offs
     // Groups as for the CELT frame kernel: the serial LPC phase of one group's CTAs then overlaps the parallel phases of the
     // others'.  A timed pass launches the SILK frame kernel once.
     const int G = b->timing ? 1 : frame_groups(b, !d_stream_idx);
-    return frame_launches(b, p, G, [&](int g, cudaStream_t st) {
+    rc = frame_launches(b, p, G, [&](int g, cudaStream_t st) {
         a.item0 = group_first(n_items, g, G);
         a.item_end = group_first(n_items, g + 1, G);
         return launch_silk_frame(a, st);
     });
+    if (rc) return rc;
+    b->mode_pending = true;
+    return OPN_OK;
 }
 
-int mix_alloc(opn_batch *b)
+int mix_alloc(opn_batch *b, bool modes)
 {
+    if (modes && !b->d_mix_sitems[0]) {
+        const size_t n = b->n, scap = mix_silk_cap(b->n);
+        for (int q = 0; q < opn_batch::NSETS; q++) {
+            CU(cudaMalloc(&b->d_mix_sitems[q], 3 * scap * sizeof(uint32_t)));
+            CU(cudaMalloc(&b->d_mix_sms[q], scap));
+            CU(cudaMalloc(&b->d_mix_sw[q], 2 * n * sizeof(uint32_t)));
+            CU(cudaMalloc(&b->d_shdr[q], n * sizeof(uint4)));
+            CU(cudaMalloc(&b->d_sstatus[q], n * sizeof(int32_t)));
+        }
+    }
     if (b->d_last_lm) return OPN_OK;
     const size_t n = b->n, cap = mix_item_cap(b->n);
     CU(cudaMalloc(&b->d_mix_key, n));
-    CU(cudaMalloc(&b->d_mix_rank, n * sizeof(uint32_t)));
+    CU(cudaMalloc(&b->d_mix_rank, 2 * n * sizeof(uint32_t)));
     for (int q = 0; q < opn_batch::NSETS; q++) {
         CU(cudaMalloc(&b->d_mix_items[q], 3 * cap * sizeof(uint32_t)));
         CU(cudaMalloc(&b->d_mix_lm[q], cap));
@@ -540,11 +568,14 @@ int mix_alloc(opn_batch *b)
 // One step whose streams may have different frame sizes (device-resident: one single-frame packet or a loss per stream).
 // The step's buckets are built on the device, so the host never learns the sizes: the range decode is ONE launch over the
 // padded item table, the frame kernel one k_frame_mix launch per group, each sized by its upper bound.
+// modes (OPN_FLAG_MIXED_MODES): SILK packets too, and mode switches.  Then the SILK range decode follows the CELT one on the
+// range-decode stream, over the SILK item table, and each group's frame stream runs: k_mode_switch (resets), k_frame_mix
+// (with the CELT -> SILK concealment items), the SILK frame kernel, k_mode_switch (the fade, when there are dense rows).
 int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, const uint32_t *d_lens, size_t capacity, float *dense,
-              size_t dense_stride, int32_t *d_result, int inputs_on, bool softclip_reset)
+              size_t dense_stride, int32_t *d_result, int inputs_on, bool softclip_reset, bool modes = false)
 {
     Range nv("opn: mixed-frame step (bucketing + range decode + frame kernel)");
-    int rc = mix_alloc(b);
+    int rc = mix_alloc(b, modes);
     if (rc) return rc;
     const int p = begin_step(b, true, inputs_on);
     if (p < 0) return p;
@@ -567,6 +598,15 @@ int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, c
     x.item_stream = b->d_mix_items[p] + 2 * (size_t)cap;
     x.item_lm = b->d_mix_lm[p];
     x.result = d_result;
+    const uint32_t scap = mix_silk_cap(b->n);
+    if (modes) {
+        x.modes = b->cfg.bitstream == OPN_BITSTREAM_OPUS ? 2 : 1;
+        x.sitem_offsets = b->d_mix_sitems[p];
+        x.sitem_lens = b->d_mix_sitems[p] + scap;
+        x.sitem_stream = b->d_mix_sitems[p] + 2 * (size_t)scap;
+        x.sitem_ms = b->d_mix_sms[p];
+        x.sw = b->d_mix_sw[p];
+    }
     SymbolArgs s{};
     s.arena = d_arena;
     s.offsets = x.item_offsets;
@@ -607,7 +647,14 @@ int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, c
     m.hist_samples = b->timing ? b->d_hist_samples : nullptr;
     m.plan = b->d_mix_plan[p];
     x.pf = nullptr;
-    if (b->lm_pending) {  // k_mix_key takes the frame sizes from the post-filter state, after the other steps' frame kernels
+    if (modes && (b->mode_pending || b->lm_pending)) {  // the same, for sizes and codecs, after the last step's frame kernels
+        const int q = b->fr_set;
+        CU(cudaStreamWaitEvent(mix_stream(b), b->ev_k1[q], 0));
+        if (b->k1_grouped[q])
+            for (int g = 1; g < opn_batch::NGROUPS; g++) CU(cudaStreamWaitEvent(mix_stream(b), b->ev_fr[q][g], 0));
+        x.pf = b->d_pf;
+        b->lm_pending = b->mode_pending = false;
+    } else if (!modes && b->lm_pending) {  // k_mix_key takes the frame sizes from the post-filter state, after the other steps' frame kernels
         const int q = b->lm_set;
         CU(cudaStreamWaitEvent(mix_stream(b), b->ev_k1[q], 0));
         if (b->k1_grouped[q])
@@ -621,17 +668,76 @@ int run_mixed(opn_batch *b, const uint8_t *d_arena, const uint32_t *d_offsets, c
     if (rc) return rc;
     rc = range_decode(b, p, [&](cudaStream_t st) { return celt2 ? launch_celt2_rangedec(s, st) : launch_synth_rangedec(s, st); });
     if (rc) return rc;
-    return frame_launches(b, p, G, [&](int g, cudaStream_t st) {
-        m.group = g;
-        return launch_frame_mix(m, group_first(b->n, g + 1, G) - group_first(b->n, g, G), st);
+    if (!modes)
+        return frame_launches(b, p, G, [&](int g, cudaStream_t st) {
+            m.group = g;
+            return launch_frame_mix(m, group_first(b->n, g + 1, G) - group_first(b->n, g, G), st);
+        });
+    SilkArgs a{};
+    a.arena = d_arena;
+    a.offsets = x.sitem_offsets;
+    a.lens = x.sitem_lens;
+    a.stream_idx = x.sitem_stream;
+    a.item_ms = x.sitem_ms;
+    a.plan = b->d_mix_plan[p];
+    a.n_items = scap;
+    a.stream_channels = b->cfg.channels;
+    a.channels = b->cfg.channels;
+    a.has_toc = 1;
+    a.bandwidth = -1;
+    a.rec = b->d_silk_rec[p];
+    a.hdr = b->d_shdr[p];
+    a.status = b->d_sstatus[p];
+    a.st = b->d_silk;
+    a.ring = b->d_ring;
+    a.ring_pos = b->d_ring_pos;
+    a.dense = dense;
+    a.dense_stride = dense_stride;
+    a.gain = b->gain;
+    a.result = d_result;
+    a.final_range = b->d_final;
+    a.softclip_reset = m.softclip_reset;
+    a.pf = b->d_pf;
+    rc = range_decode(b, p, [&](cudaStream_t st) { return launch_silk_rangedec(a, st); });
+    if (rc) return rc;
+    SwitchArgs w{};
+    w.plan = b->d_mix_plan[p];
+    w.channels = b->cfg.channels;
+    w.sw = x.sw;
+    w.n_streams = b->n;
+    w.carry = b->d_carry;
+    w.ring = b->d_ring;
+    w.ring_pos = b->d_ring_pos;
+    w.pf = b->d_pf;
+    w.silk_fs = b->d_silk.fs;
+    w.dense = dense;
+    w.dense_stride = dense_stride;
+    w.gain = b->gain;
+    rc = frame_launches(b, p, G, [&](int g, cudaStream_t st) {
+        const uint32_t ng = group_first(b->n, g + 1, G) - group_first(b->n, g, G);
+        w.group = m.group = a.group = g;
+        w.first = group_first(b->n, g, G);
+        w.phase = 0;
+        cudaError_t e = launch_mode_switch(w, ng, st);
+        if (e == cudaSuccess) e = launch_frame_mix(m, ng, st);
+        if (e == cudaSuccess) e = launch_silk_frame_mix(a, ng, st);
+        w.phase = 1;
+        if (e == cudaSuccess && dense) e = launch_mode_switch(w, ng, st);
+        b->launches[1]++;  // frame_launches counts the CELT frame kernel, this the SILK one
+        b->launches[2] += dense ? 2 : 1;
+        return e;
     });
+    if (rc) return rc;
+    b->silk_dev = true;
+    return OPN_OK;
 }
 
 // Device-resident steps keep what the host path conceals with on the device: a stream's frame size in PfState::lm1, the
 // rate and coded channels of its last SILK frame in the SILK state.  Before the first host-buffer call after such steps,
-// the host mirrors are brought up to date from there.  Device-resident steps do not switch a stream between CELT and
-// SILK, so a stream that already has a mode keeps it; one that had none takes SILK when a SILK frame was decoded, CELT
-// when a CELT frame kernel recorded a size.
+// the host mirrors are brought up to date from there.  Uniform and mixed-frame steps do not switch a stream between CELT
+// and SILK, so a stream that already has a mode keeps it; one that had none takes SILK when a SILK frame was decoded, CELT
+// when a CELT frame kernel recorded a size.  After mixed-mode steps, which do switch, every stream whose record holds a
+// packet takes its codec from the record (PF_SILK).
 int sync_host_state(opn_batch *b)
 {
     if (!b->dev_steps) return OPN_OK;
@@ -645,11 +751,16 @@ int sync_host_state(opn_batch *b)
     CU(cudaStreamSynchronize(b->stream));
     for (size_t i = 0; i < n; i++) {
         const bool silk_frame = b->silk && fs[2 * i] != 0;
-        if (!b->have_mode[i] && (silk_frame || pf[i].lm1 > 0)) b->have_mode[i] = 1 + (silk_frame ? OPN_MODE_SILK : OPN_MODE_CELT);
+        const int32_t l1 = pf[i].lm1 & PF_LM1;
+        const bool silk_rec = (pf[i].lm1 & PF_SILK) != 0;  // the last packet was SILK (a PLC/DTX one too)
+        if (b->silk_dev && l1 > 0) b->have_mode[i] = 1 + (silk_rec ? OPN_MODE_SILK : OPN_MODE_CELT);
+        if (!b->have_mode[i] && (silk_frame || l1 > 0)) b->have_mode[i] = 1 + (silk_frame || silk_rec ? OPN_MODE_SILK : OPN_MODE_CELT);
         if (silk_frame && b->have_mode[i] == 1 + OPN_MODE_SILK) b->silk_cs[i] = fs[2 * i + 1];
-        if (pf[i].lm1 > 0) b->last_nf[i] = 120 << (pf[i].lm1 - 1);
+        // a stream concealed as silence before its first SILK frame: device-resident SILK packets have the batch's channels
+        if (b->have_mode[i] == 1 + OPN_MODE_SILK && b->silk_cs[i] == 0) b->silk_cs[i] = (uint8_t)b->cfg.channels;
+        if (l1 > 0) b->last_nf[i] = 120 << (l1 - 1);
     }
-    b->dev_steps = false;
+    b->dev_steps = b->silk_dev = false;
     return OPN_OK;
 }
 
@@ -877,6 +988,11 @@ void opn_batch_destroy(opn_batch *b)
         cudaFree(b->d_mix_items[q]);
         cudaFree(b->d_mix_lm[q]);
         cudaFree(b->d_mix_plan[q]);
+        cudaFree(b->d_mix_sitems[q]);
+        cudaFree(b->d_mix_sms[q]);
+        cudaFree(b->d_mix_sw[q]);
+        cudaFree(b->d_shdr[q]);
+        cudaFree(b->d_sstatus[q]);
         if (b->ev_mix[q]) cudaEventDestroy(b->ev_mix[q]);
     }
     cudaFree(b->d_hist_samples);
@@ -919,7 +1035,7 @@ int opn_batch_reset(opn_batch *b)  // DecoderInner::reset, decoder.rs:286-303, f
     b->set = 0;
     CU(cudaMemsetAsync(b->d_softclip, 0, n * 2 * sizeof(float), b->stream));
     if (b->d_last_lm) CU(cudaMemsetAsync(b->d_last_lm, MIX_NO_ITEM, n, b->stream));
-    b->lm_pending = false;
+    b->lm_pending = b->mode_pending = false;
     if (b->silk) {
         CU(cudaMemsetAsync(b->d_silk.slpc, 0, n * 2 * 16 * sizeof(int32_t), b->stream));
         CU(cudaMemsetAsync(b->d_silk.hist, 0, n * 2 * SILK_HIST * sizeof(int32_t), b->stream));
@@ -934,7 +1050,7 @@ int opn_batch_reset(opn_batch *b)  // DecoderInner::reset, decoder.rs:286-303, f
     std::fill(b->last_duration.begin(), b->last_duration.end(), -1);
     std::fill(b->have_mode.begin(), b->have_mode.end(), 0);
     std::fill(b->silk_cs.begin(), b->silk_cs.end(), 0);
-    b->dev_steps = false;
+    b->dev_steps = b->silk_dev = false;
     return OPN_OK;
 }
 
@@ -1244,7 +1360,7 @@ int opn_batch_decode_float(opn_batch *b, const uint8_t *arena, const uint32_t *o
     const int C = b->cfg.channels;
     CU(cudaSetDevice(b->device));
     if (!(flags & OPN_FLAG_DEVICE_PTRS)) {
-        if (!arena) return OPN_ERR_BAD_ARG;
+        if (!arena || (flags & OPN_FLAG_MIXED_MODES)) return OPN_ERR_BAD_ARG;
         if (pcm && pcm_stride_floats < frame_size * (size_t)C) return OPN_ERR_BUFFER_TOO_SMALL;
         const int rc = batch_decode_host(b, arena, offsets, lens, pcm, pcm_stride_floats, frame_size, result_per_stream, flags);
         if (rc < 0) return rc;
@@ -1255,7 +1371,9 @@ int opn_batch_decode_float(opn_batch *b, const uint8_t *arena, const uint32_t *o
     // frame_size samples; with it frame_size is the capacity of a stream's row, as in decode_float, and each stream
     // decodes whatever single frame its packet holds.
     if (!arena) return OPN_ERR_BAD_ARG;
-    if (b->cfg.bitstream == OPN_BITSTREAM_OPUS && !(flags & OPN_FLAG_SILK_FRAMES)) return OPN_ERR_UNIMPLEMENTED;  // celt/decoder.rs:47-56 is todo!()
+    if ((flags & OPN_FLAG_MIXED_MODES) && (!b->silk || (flags & OPN_FLAG_SILK_FRAMES))) return OPN_ERR_BAD_ARG;
+    // celt/decoder.rs:47-56 is todo!(); a mixed-mode step reports the CELT packets per stream
+    if (b->cfg.bitstream == OPN_BITSTREAM_OPUS && !(flags & (OPN_FLAG_SILK_FRAMES | OPN_FLAG_MIXED_MODES))) return OPN_ERR_UNIMPLEMENTED;
     b->dev_steps = true;
     float *dense = (flags & OPN_FLAG_NO_PCM_COPY) ? nullptr : pcm;
     if (dense && (pcm_stride_floats < std::min<size_t>(frame_size, 960) * (size_t)C || (pcm_stride_floats & 3) ||
@@ -1267,9 +1385,9 @@ int opn_batch_decode_float(opn_batch *b, const uint8_t *arena, const uint32_t *o
         return run_silk_bucket(b, arena, offsets, lens, nullptr, nullptr, b->n, frame_size == 960 ? 20 : 10, 1, -1, C, dense, pcm_stride_floats,
                                result_per_stream, (flags & OPN_FLAG_INPUTS_READY) ? 0 : 1, true);
     }
-    if (flags & OPN_FLAG_MIXED_FRAMES)
+    if (flags & (OPN_FLAG_MIXED_FRAMES | OPN_FLAG_MIXED_MODES))
         return run_mixed(b, arena, offsets, lens, frame_size, dense, pcm_stride_floats, result_per_stream,
-                         (flags & OPN_FLAG_INPUTS_READY) ? 0 : 1, true);
+                         (flags & OPN_FLAG_INPUTS_READY) ? 0 : 1, true, (flags & OPN_FLAG_MIXED_MODES) != 0);
     const int lm = lm_of_frame(frame_size);
     if (lm < 0) return OPN_ERR_BAD_ARG;
     if (dense && pcm_stride_floats < frame_size * (size_t)C) return OPN_ERR_BAD_ARG;
@@ -1296,7 +1414,7 @@ int opn_batch_decode_pcm(opn_batch *b, const uint8_t *arena, const uint32_t *off
     if (!b || !arena || !offsets || !lens || !pcm) return OPN_ERR_BAD_ARG;
     if (opn_sample_size(sample_format) == 0) return OPN_ERR_BAD_ARG;
     if (frame_size == 0 || frame_size % 120 != 0) return OPN_ERR_BAD_ARG;  // decoder.rs:316-320
-    if (flags & (OPN_FLAG_DEVICE_PTRS | OPN_FLAG_NO_PCM_COPY)) return OPN_ERR_BAD_ARG;
+    if (flags & (OPN_FLAG_DEVICE_PTRS | OPN_FLAG_NO_PCM_COPY | OPN_FLAG_MIXED_MODES)) return OPN_ERR_BAD_ARG;
     if (pcm_stride_samples < frame_size * (size_t)b->cfg.channels) return OPN_ERR_BUFFER_TOO_SMALL;
     if (frame_size * (size_t)b->cfg.channels * sizeof(float) > 200 * 1024) return OPN_ERR_BAD_ARG;  // the clip epilogue stages a row on chip
     CU(cudaSetDevice(b->device));

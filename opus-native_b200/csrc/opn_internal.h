@@ -33,9 +33,12 @@ struct PfState {  // post-filter parameters of the previous frame
     float gain;
     // 1 + LM of the frame size the stream conceals a loss with, 0 = no packet yet: the size of its last frame that came from
     // a packet, decoded or PLC/DTX (a TOC with a payload of at most one byte: libopus takes st->frame_size from the TOC
-    // before it decodes the frames).  Written by every CELT frame kernel and by the SILK frame kernel (960 -> 4, 480 -> 3).
+    // before it decodes the frames).  Written by every CELT frame kernel and by the SILK frame kernel (960 -> 4, 480 -> 3),
+    // which also sets PF_SILK: the codec of that packet.  Every reader masks it off (PF_LM1).
     int32_t lm1;
 };
+// The codec bit of a stream's mode record: in PfState::lm1 (OR-ed onto 1 + LM) and in the mixed steps' last_lm (OR-ed onto LM).
+constexpr int32_t PF_SILK = 0x40, PF_LM1 = 0x0F;
 
 // Frame header, range decode -> frame kernel: one uint4 per stream.
 //   .x = silence | postfilter << 1 | transient << 2 | intra << 3 | tapset << 4 | gain_idx << 8 | octave << 12 | period << 16
@@ -66,8 +69,17 @@ struct MixPlan {
     uint32_t start[MIX_GROUPS][4];
     uint32_t cta0[MIX_GROUPS][5];  // frame kernel: first CTA of group g's j-th bucket (lm = 3 - j: longest frames first); [4] = CTAs in use
     uint32_t items_padded;         // items up to the end of the last bucket
+    // mixed-mode steps (OPN_FLAG_MIXED_MODES) only.  SILK bucket (g, k), k = 0 for 10 ms and 1 for 20 ms, owns the items
+    // [sstart, sstart + scount) of the SILK item table; each starts on a multiple of SILK_PAD items, so that one SILK frame CTA
+    // never spans two durations.  The CELT->SILK streams' 2.5 ms concealments are items of the CELT bucket (g, 1).
+    uint32_t scount[MIX_GROUPS][2];
+    uint32_t sstart[MIX_GROUPS][2];
+    uint32_t scta0[MIX_GROUPS][3];  // SILK frame kernel: first CTA of group g's j-th bucket (k = 1 - j: 20 ms first); [2] = CTAs in use
+    uint32_t nsw[MIX_GROUPS][2];    // streams of group g that switch [0] CELT -> SILK, [1] SILK -> CELT (listed in MixArgs::sw)
 };
 __host__ __device__ constexpr uint32_t mix_item_cap(uint32_t n_streams) { return n_streams + MIX_GROUPS * 4u * MIX_PAD; }
+constexpr uint32_t SILK_PAD = 32u;
+__host__ __device__ constexpr uint32_t mix_silk_cap(uint32_t n_streams) { return n_streams + MIX_GROUPS * 2u * SILK_PAD; }
 
 struct SymbolArgs {
     const uint8_t *arena;
@@ -124,12 +136,33 @@ struct MixArgs {  // k_mix_key / k_mix_place
     uint32_t capacity;               // samples per channel the caller's rows hold (frame_size argument)
     uint8_t *last_lm;                // [n_streams] LM of the stream's last packet (decoded or PLC/DTX), MIX_NO_ITEM = none yet (state)
     const PfState *pf;               // [n_streams] or nullptr: after other CELT steps, last_lm is first taken from PfState::lm1
-    uint8_t *key;                    // [n_streams] scratch: g*4 + lm, or MIX_NO_ITEM
-    uint32_t *rank;                  // [n_streams] scratch: position inside the bucket
+    uint8_t *key;                    // [n_streams] scratch: g*4 + lm, MIX_KEY_SILK | g*2 + k (| MIX_KEY_TRANS), or MIX_NO_ITEM
+    uint32_t *rank;                  // [2 n_streams] scratch: position inside the bucket; [n_streams + s]: of the transition item
     MixPlan *plan;                   // zeroed before k_mix_key
     uint32_t *item_offsets, *item_lens, *item_stream;  // [mix_item_cap] out
     uint8_t *item_lm;                // [mix_item_cap] out, preset to MIX_NO_ITEM
     int32_t *result;                 // [n_streams] or nullptr: OPN_ERR_* of the streams no bucket takes
+    // mixed-mode step (OPN_FLAG_MIXED_MODES): SILK packets are bucketed too, and mode switches listed
+    int modes;                       // 0: CELT-only step (SILK packets are errors); 1: CELT and SILK; 2: SILK only (CELT packets are errors)
+    uint32_t *sitem_offsets, *sitem_lens, *sitem_stream;  // [mix_silk_cap] out: the SILK item table
+    uint8_t *sitem_ms;               // [mix_silk_cap] out, preset to MIX_NO_ITEM: frame duration of the SILK item (10 / 20)
+    uint32_t *sw;                    // [2][n_streams] out: switch d of group g is listed at sw[d n + group_first(g) + k], k < nsw[g][d]
+};
+constexpr uint8_t MIX_KEY_SILK = 0x20, MIX_KEY_TRANS = 0x40;
+
+// The mode switches of one group of a mixed-mode step, before (phase 0: resets) and after (phase 1: fade) its frame kernels.
+struct SwitchArgs {
+    const MixPlan *plan;
+    int group, phase, channels;
+    const uint32_t *sw;          // MixArgs::sw
+    uint32_t n_streams, first;   // first = group_first(n_streams, group)
+    float *carry, *ring;
+    uint32_t *ring_pos;
+    PfState *pf;
+    uint8_t *silk_fs;            // SilkState::fs
+    float *dense;                // or nullptr: no fade
+    size_t dense_stride;
+    float gain;
 };
 
 // ---- SYNTH-SILK/1 (silk.cuh; DESIGN.md section 3c)
@@ -190,6 +223,9 @@ struct SilkArgs {
     int32_t *exc_out;      // [n_streams][2][SILK_MAX_FRAME] or nullptr
     int16_t *out16;        // [n_streams][2][SILK_MAX_FRAME] or nullptr
     unsigned long long *phase_clk;  // measurement (OPN_SILK_CLK=1): [3] cycles in phases A, B, C summed over CTAs, [3] = CTAs; else nullptr
+    const uint8_t *item_ms;    // mixed-mode step: [n_items] frame duration of the item, MIX_NO_ITEM = padding (overrides frame_ms); else nullptr
+    const MixPlan *plan;       // mixed-mode step: the frame kernel's CTAs find their bucket here (item0 / item_end / frame_ms unused)
+    int group;
 };
 
 // ---- launchers (opn_kernels.cu).  All return a cudaError_t and never synchronise.
@@ -207,10 +243,13 @@ cudaError_t launch_frame(const FrameArgs &a, cudaStream_t st);
 // mixed-frame step: bucketing (two kernels on one stream) and the frame kernel of one group (a.plan, a.group; grid sized by the
 // caller's upper bound n_streams_in_group)
 cudaError_t launch_mix_plan(const MixArgs &a, cudaStream_t st);
+cudaError_t launch_mode_switch(const SwitchArgs &a, uint32_t n_streams_in_group, cudaStream_t st);  // k_mode_switch
 cudaError_t launch_op_smooth_fade(const float *in1, const float *in2, float *out, size_t row_stride, int overlap, int channels, int fs,
                                   uint32_t n_rows, cudaStream_t st);
 cudaError_t launch_silk_rangedec(const SilkArgs &a, cudaStream_t st);  // one lane per packet -> one record per coded channel
 cudaError_t launch_silk_frame(const SilkArgs &a, cudaStream_t st);     // excitation + LTP + LPC synthesis + resampler + PCM store
+// mixed-mode step: the SILK frame kernel of one group (a.plan, a.group), grid sized by the group's upper bound
+cudaError_t launch_silk_frame_mix(const SilkArgs &a, uint32_t n_streams_in_group, cudaStream_t st);
 cudaError_t launch_transition_fade(float *dense, size_t dense_stride, const uint32_t *d_streams, uint32_t n_streams, uint32_t n_rows, int channels,
                                    cudaStream_t st);  // CELT -> SILK: 2.5 ms of the old decoder's concealment, then a 2.5 ms cross-fade
 int kernels_frame_groups();  // OPN_FRAME_GROUPS the kernels were built with

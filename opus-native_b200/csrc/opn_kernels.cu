@@ -304,6 +304,8 @@ cudaError_t upload_tables(int device)
         if (e == cudaSuccess) e = cudaFuncSetAttribute(k_silk_frame<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)silk_frame_smem());
         if (e == cudaSuccess) e = cudaFuncSetAttribute(k_silk_frame<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)silk_frame_smem());
         if (e == cudaSuccess) e = cudaFuncSetAttribute(k_silk_frame<2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)silk_frame_smem());
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_silk_frame<1, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)silk_frame_smem());
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_silk_frame<2, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)silk_frame_smem());
     }
     if (e != cudaSuccess) return e;
     e = set_warp_kernel_attributes();
@@ -429,12 +431,25 @@ cudaError_t launch_mix_plan(const MixArgs &a, cudaStream_t st)
     if (a.n_streams == 0) return cudaSuccess;
     if (!a.plan || !a.key || !a.rank || !a.last_lm || !a.item_lm || !a.item_offsets || !a.item_lens || !a.item_stream) return cudaErrorInvalidValue;
     if (a.n_groups != 1 && a.n_groups != MIX_GROUPS) return cudaErrorInvalidValue;
+    if (a.modes && (!a.sitem_offsets || !a.sitem_lens || !a.sitem_stream || !a.sitem_ms || !a.sw))
+        return cudaErrorInvalidValue;
     cudaError_t e = cudaMemsetAsync(a.plan, 0, sizeof(MixPlan), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(a.item_lm, MIX_NO_ITEM, mix_item_cap(a.n_streams), st);
+    if (e == cudaSuccess && a.modes) e = cudaMemsetAsync(a.sitem_ms, MIX_NO_ITEM, mix_silk_cap(a.n_streams), st);
     if (e != cudaSuccess) return e;
     const uint32_t grid = (a.n_streams + 255u) / 256u;
     k_mix_key<<<grid, 256, 0, st>>>(a);
     k_mix_place<<<grid, 256, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_mode_switch(const SwitchArgs &a, uint32_t n_streams_in_group, cudaStream_t st)
+{
+    if (n_streams_in_group == 0) return cudaSuccess;
+    if (!a.plan || !a.sw || a.group < 0 || a.group >= MIX_GROUPS || (a.phase == 1 && !a.dense)) return cudaErrorInvalidValue;
+    // one warp per switching stream: a few percent of the group's streams switch in a step
+    const uint32_t grid = std::min<uint32_t>((n_streams_in_group + 63u) / 64u, 256u);
+    k_mode_switch<<<grid, 256, 0, st>>>(a);
     return cudaGetLastError();
 }
 
@@ -596,6 +611,18 @@ cudaError_t launch_silk_frame(const SilkArgs &a0, cudaStream_t st)
     else if (cs == 1) k_silk_frame<1, 2><<<grid, 32 * SILK_WARPS, smem, st>>>(a);
     else if (c == 1) k_silk_frame<2, 1><<<grid, 32 * SILK_WARPS, smem, st>>>(a);
     else k_silk_frame<2, 2><<<grid, 32 * SILK_WARPS, smem, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_silk_frame_mix(const SilkArgs &a, uint32_t n_streams_in_group, cudaStream_t st)
+{
+    if (n_streams_in_group == 0) return cudaSuccess;
+    if (!a.plan || a.group < 0 || a.group >= MIX_GROUPS || !a.stream_idx || a.stream_channels != a.channels) return cudaErrorInvalidValue;
+    const uint32_t per_cta = (uint32_t)(SILK_ROWS / a.stream_channels);
+    const uint32_t grid = (n_streams_in_group + per_cta - 1u) / per_cta + 2u;  // each of the two buckets rounds up
+    const size_t smem = silk_frame_smem();
+    if (a.channels == 1) k_silk_frame<1, 1, true><<<grid, 32 * SILK_WARPS, smem, st>>>(a);
+    else k_silk_frame<2, 2, true><<<grid, 32 * SILK_WARPS, smem, st>>>(a);
     return cudaGetLastError();
 }
 

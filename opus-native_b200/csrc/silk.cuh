@@ -55,6 +55,11 @@ __global__ void __launch_bounds__(32) k_silk_rangedec(SilkArgs A)
     __syncwarp();
     const uint32_t item = blockIdx.x * 32u + lane;
     if (item >= A.n_items) return;
+    int frame_ms = A.frame_ms;
+    if (A.item_ms) {  // mixed-mode step: padding items between the buckets
+        frame_ms = A.item_ms[item];
+        if (frame_ms == MIX_NO_ITEM) return;
+    }
     const uint32_t stream = A.stream_idx ? A.stream_idx[item] : item;
     uint32_t len = A.lens[item];
     const uint8_t *src = A.arena + A.offsets[item];
@@ -67,7 +72,7 @@ __global__ void __launch_bounds__(32) k_silk_rangedec(SilkArgs A)
         if (config >= 12u) status = OPN_ERR_UNIMPLEMENTED;                                  // hybrid / CELT: not this launch
         else if ((toc & 0x3u) != 0u) status = OPN_ERR_UNIMPLEMENTED;                        // multi-frame: host path only
         else if ((config & 3u) > 1u) status = OPN_ERR_UNIMPLEMENTED;                        // 40 / 60 ms: several SILK frames
-        else if ((int)((config & 3u) ? 20 : 10) != A.frame_ms) status = OPN_ERR_FRAME_SIZE_TOO_SMALL;
+        else if ((int)((config & 3u) ? 20 : 10) != frame_ms) status = OPN_ERR_FRAME_SIZE_TOO_SMALL;
         else if (((toc & 0x4u) ? 2 : 1) != A.stream_channels) status = OPN_ERR_UNIMPLEMENTED;
         bandwidth = (int)(config >> 2);
         src += 1;
@@ -80,7 +85,7 @@ __global__ void __launch_bounds__(32) k_silk_rangedec(SilkArgs A)
         return;
     }
     const int fs_khz = bandwidth == 0 ? 8 : bandwidth == 1 ? 12 : 16;
-    const int nb_subfr = A.frame_ms / 5, order = fs_khz == 16 ? 16 : 10, nblk = (nb_subfr * 5 * fs_khz + 15) / 16;
+    const int nb_subfr = frame_ms / 5, order = fs_khz == 16 ? 16 : 10, nblk = (nb_subfr * 5 * fs_khz + 15) / 16;
     const int min_lag = 2 * fs_khz, max_lag = 18 * fs_khz;
     const PvqTable T{g_tab.pvq_u_data, g_tab.pvq_u_row};
     LaneDec d;
@@ -222,7 +227,8 @@ __device__ __forceinline__ void silk_resample_store(const float *x, int L, uint3
     }
 }
 
-template <int CS, int C> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k_silk_frame(SilkArgs A)
+// MIX: a mixed-mode step's launch (A.plan); a separate instance, so that the uniform and host-path launches keep their registers
+template <int CS, int C, bool MIX = false> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k_silk_frame(SilkArgs A)
 {
     extern __shared__ __align__(16) uint8_t silk_smem[];
     // [SILK_LEAD + SILK_MAX_FRAME][SILK_RS]: excitation, then internal-rate samples (as floats); s_res points at sample 0
@@ -235,8 +241,19 @@ template <int CS, int C> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     const long long clk0 = A.phase_clk ? clock64() : 0;
     constexpr uint32_t ITEMS = SILK_ROWS / CS;
-    const uint32_t item0 = A.item0 + blockIdx.x * ITEMS;
-    const int nb_subfr = A.frame_ms / 5;
+    uint32_t item0 = A.item0 + blockIdx.x * ITEMS, item_end = A.item_end;
+    int frame_ms = A.frame_ms;
+    if constexpr (MIX) {  // mixed-mode step: the CTA's bucket (20 ms first); the grid is an upper bound, CTAs past the last bucket retire
+        const MixPlan &P = *A.plan;
+        const int g = A.group;
+        const uint32_t c = blockIdx.x;
+        if (c >= P.scta0[g][2]) return;
+        const int j = c >= P.scta0[g][1], k = 1 - j;
+        frame_ms = k ? 20 : 10;
+        item0 = P.sstart[g][k] + (c - P.scta0[g][j]) * ITEMS;
+        item_end = P.sstart[g][k] + P.scount[g][k];
+    }
+    const int nb_subfr = frame_ms / 5;
 
     // ---- phase A0: one thread per row: what the row is (frame parameters, where its state lives)
     __shared__ uint32_t s_chs[SILK_ROWS];  // stream * 2 + coded channel
@@ -245,7 +262,7 @@ template <int CS, int C> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k
         uint8_t *meta = s_meta + row * 8;
         meta[0] = 0;
         meta[3] = 3;  // no item
-        if (item < A.item_end) {
+        if (item < item_end) {
             const uint32_t stream = A.stream_idx ? A.stream_idx[item] : item;
             const int32_t status = A.status[stream];
             const uint32_t fs_prev = A.st.fs[2 * stream], cs_prev = A.st.fs[2 * stream + 1];
@@ -478,10 +495,10 @@ template <int CS, int C> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k
     // ---- phase C: one warp per item
     for (uint32_t it = warp; it < ITEMS; it += SILK_WARPS) {
         const uint32_t item = item0 + it;
-        if (item >= A.item_end) continue;
+        if (item >= item_end) continue;
         const uint32_t row0 = it * CS;
         const uint32_t stream = A.stream_idx ? A.stream_idx[item] : item;
-        const int n48 = A.frame_ms * 48;
+        const int n48 = frame_ms * 48;
         const uint32_t flag = s_meta[row0 * 8 + 3];
         const uint32_t dense_off = (A.dense && A.dense_off) ? A.dense_off[item] : 0u;
         float *dense = A.dense ? A.dense + (size_t)stream * A.dense_stride + dense_off : nullptr;
@@ -495,6 +512,8 @@ template <int CS, int C> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k
             if (lane == 0) {
                 if (A.result) A.result[stream] = n48;
                 if (A.final_range) A.final_range[stream] = 0u;
+                // a PLC/DTX packet still sets the stream's codec and size (the mode record of mixed-mode steps)
+                if (A.pf && (A.hdr[stream].x & HDR_DTX)) A.pf[stream].lm1 = (nb_subfr == 4 ? 4 : 3) | PF_SILK;
             }
             continue;
         }
@@ -541,7 +560,7 @@ template <int CS, int C> __global__ void __launch_bounds__(32 * SILK_WARPS, 4) k
                 A.st.fs[2 * stream] = (uint8_t)fs_khz;
                 A.st.fs[2 * stream + 1] = (uint8_t)CS;
             }
-            if (A.pf && (!lost || (A.hdr[stream].x & HDR_DTX))) A.pf[stream].lm1 = nb_subfr == 4 ? 4 : 3;
+            if (A.pf && (!lost || (A.hdr[stream].x & HDR_DTX))) A.pf[stream].lm1 = (nb_subfr == 4 ? 4 : 3) | PF_SILK;
             if (A.result) A.result[stream] = n48;
             if (A.final_range) A.final_range[stream] = lost ? 0u : A.hdr[stream].y;
             if (A.softclip_reset && !lost) *reinterpret_cast<float2 *>(A.softclip_reset + 2 * (size_t)stream) = make_float2(0.f, 0.f);
