@@ -17,19 +17,19 @@ class MixedModeBatch:
         whose first 2.5 ms replace the start of the SILK frame and whose next 2.5 ms cross-fade into it (smooth_fade);
       - CELT after SILK: the CELT decoder starts from rest;
       - a loss conceals one frame of the stream's last size with the codec of its last packet; before any packet, one CELT
-        frame of the row's capacity (zeros).  A PLC/DTX packet (lens 1 or 2) sets codec and size from its TOC.
+        frame of the step's row capacity (zeros).  A PLC/DTX packet (lens 1 or 2) sets codec and size from its TOC.
     Built on CeltBatch / SilkBatch steps with skip and on resets of single states, so it runs at tens of thousands of streams.
     Stream s decodes exactly as one SynthStream / Celt2Stream and one SilkStream composed by hand would."""
 
-    def __init__(self, n_streams, channels, bitstream=1, cap=960, n_threads=None):
-        """bitstream: the CELT layout, 1 or 2; 0 (OPN_BITSTREAM_OPUS): CELT packets are rejected (OPN_ERR_UNIMPLEMENTED)"""
+    def __init__(self, n_streams, channels, bitstream=1, cap=960, n_threads=None, apply_comb=True):
+        """bitstream: the CELT layout, 1 or 2; 0 (OPN_BITSTREAM_OPUS): CELT packets are rejected (OPN_ERR_UNIMPLEMENTED).
+        apply_comb: the CELT post-filter (a batch created with postfilter = false runs without it)"""
         self.n, self.channels, self.cap, self.celt_ok = n_streams, channels, cap, bitstream != 0
-        self.celt = CeltBatch(n_streams, channels, bitstream or 1, n_threads=n_threads)
+        self.celt = CeltBatch(n_streams, channels, bitstream or 1, apply_comb=apply_comb, n_threads=n_threads)
         self.silk = SilkBatch(n_streams, channels, n_threads=n_threads)
         self.mode = np.zeros(n_streams, np.uint8)
-        cap_lm = 3 if cap >= 960 else 2 if cap >= 480 else 1 if cap >= 240 else 0
-        self.lm = np.full(n_streams, cap_lm, np.uint8)  # the size a loss conceals (LM; SILK: 2 = 10 ms, 3 = 20 ms)
-        self.final = np.zeros(n_streams, np.uint32)     # Decoder::final_range() of each stream's last decoded frame
+        self.lm = np.zeros(n_streams, np.uint8)     # the size a loss conceals once a packet was decoded (LM; SILK: 2 = 10 ms, 3 = 20 ms)
+        self.final = np.zeros(n_streams, np.uint32)  # Decoder::final_range() of each stream's last decoded frame
 
     def classify(self, packets, lens):
         """-> (codec [n]: CELT, SILK or 0 for a stream whose packet is rejected, lm [n], err [n]: OPN_ERR_* or 0), as the
@@ -38,7 +38,8 @@ class MixedModeBatch:
         toc = packets[:, 0].astype(np.int64)
         got = np.asarray(lens) > 0
         codec = np.where(self.mode == SILK, SILK, CELT).astype(np.uint8)
-        lm = self.lm.copy()
+        cap_lm = 3 if self.cap >= 960 else 2 if self.cap >= 480 else 1 if self.cap >= 240 else 0
+        lm = np.where(self.mode != 0, self.lm, cap_lm).astype(np.uint8)  # before any packet: this step's row capacity
         err = np.zeros(self.n, np.int32)
         celt = (toc & 0x80) != 0
         config = toc >> 3

@@ -14,10 +14,10 @@ def _silk_fill(first, n, frame, bw, ms, channels, nbytes):
     return O.silk_fill(first, n, frame, 1, bw, ms, channels, nbytes)[0]
 
 
-def _per_stream(packets, lens, channels, cap=960):
+def _per_stream(packets, lens, channels, cap=960, apply_comb=True):
     """-> per step (pcm [n, cap * C], result [n], final_rng [n]) from one decoder pair per stream"""
     nsteps, n = lens.shape
-    celt = [O.SynthStream(3, channels) for _ in range(n)]
+    celt = [O.SynthStream(3, channels, apply_comb) for _ in range(n)]
     silk = [O.SilkStream(channels) for _ in range(n)]
     mode = [0] * n
     last = [3] * n  # LM of the last packet; before any, the row's capacity
@@ -42,7 +42,7 @@ def _per_stream(packets, lens, channels, cap=960):
             if toc & 0x80:
                 lm = (toc >> 3) & 3
                 if mode[s] == M.SILK:
-                    celt[s] = O.SynthStream(3, channels)                    # decoder.rs:703-705
+                    celt[s] = O.SynthStream(3, channels, apply_comb)        # decoder.rs:703-705
                 celt[s].lm = lm
                 side, _, _, w = celt[s].decode(pk[1:])
                 rng[s] = side.final_rng if L > 2 else 0
@@ -73,12 +73,16 @@ def _per_stream(packets, lens, channels, cap=960):
 def test_mixed_mode_batch_equals_per_stream_composition():
     """60 streams, 16 steps: codec switches both ways, losses (some before any packet), TOC-only and one-byte packets of both
     codecs, CELT frames of 2.5-20 ms and SILK frames of every bandwidth at 10 and 20 ms."""
+    _against_per_stream(apply_comb=True)
+
+
+def _against_per_stream(apply_comb):
     rnd = np.random.default_rng(77)
     for channels in (2, 1):
         n, nsteps = 60, 16
         packets, lens = M.mixed_mode_traffic(n, nsteps, channels, rnd, _celt_fill, _silk_fill, seed=5, switch=0.2, loss=0.08, plc=0.08)
-        want = _per_stream(packets, lens, channels)
-        batch = M.MixedModeBatch(n, channels, n_threads=4)
+        want = _per_stream(packets, lens, channels, apply_comb=apply_comb)
+        batch = M.MixedModeBatch(n, channels, n_threads=4, apply_comb=apply_comb)
         switches = 0
         for f in range(nsteps):
             before = batch.mode.copy()
@@ -89,3 +93,17 @@ def test_mixed_mode_batch_equals_per_stream_composition():
             assert np.array_equal(pcm, want[f][0]), f
         assert switches > 20
         assert (lens == 1).any() and (lens == 2).any() and (lens[0] == 0).any()
+
+
+def test_mixed_mode_batch_without_post_filter_equals_per_stream_composition():
+    """apply_comb=False (a batch created with postfilter = false): the same traffic against SynthStream(apply_comb=False) and
+    SilkStream pairs, and the post-filter changes the PCM of that traffic"""
+    _against_per_stream(apply_comb=False)
+    rnd = np.random.default_rng(78)
+    packets, lens = M.mixed_mode_traffic(40, 6, 2, rnd, _celt_fill, _silk_fill, seed=6)
+    on, off = M.MixedModeBatch(40, 2, n_threads=4), M.MixedModeBatch(40, 2, n_threads=4, apply_comb=False)
+    differ = False
+    for f in range(6):
+        a, b = on.step(packets[f], lens[f])[0], off.step(packets[f], lens[f])[0]
+        differ |= not np.array_equal(a, b)
+    assert differ
